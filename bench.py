@@ -151,6 +151,26 @@ def cpu_reference_windows_per_sec(p, w, sample_windows: int, reps: int, threads:
   return sample_windows / best, best
 
 
+DUMP_LIMIT = 64 << 20   # bytes of all --dump-outputs files together
+
+
+def dump_outputs(directory: str, **arrays):
+  """--dump-outputs: each array (one row per window) as directory/<name>.npy in float32, so that two builds run with the
+  same arguments can be compared output for output.  When the windows would exceed DUMP_LIMIT, the same fixed, seeded
+  sample of windows is kept in every array and its indices are written as windows.npy (float64)."""
+  arrays = {k: np.asarray(a, np.float32) for k, a in arrays.items()}
+  n = len(next(iter(arrays.values())))
+  per_window = sum(a.nbytes for a in arrays.values()) // max(n, 1) + 8
+  keep = (DUMP_LIMIT - 4096) // per_window                      # 4 KB for the .npy headers
+  if n > keep:
+    idx = np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+    arrays = {k: a[idx] for k, a in arrays.items()}
+    arrays["windows"] = idx.astype(np.float64)
+  os.makedirs(directory, exist_ok=True)
+  for name, a in arrays.items():
+    np.save(os.path.join(directory, name + ".npy"), a)
+
+
 def run_reference(args, rank, world):
   """--impl reference: the reference's CPU path (oracle port) of the same workload on the host cores (rank 0 only).
   A step is the whole 1024-window batch, exactly as in the engine arm."""
@@ -168,13 +188,16 @@ def run_reference(args, rank, world):
 
   def step():
     out = omodel.forward(rows, p, w)
-    opost.quality_from_probs(out["probs"], 93, (cal.threshold, cal.w, cal.b))
+    return opost.quality_from_probs(out["probs"], 93, (cal.threshold, cal.w, cal.b))
   for _ in range(args.warmup):
     step()
   t0 = time.perf_counter()
   for _ in range(args.steps):
-    step()
+    y, q = step()
   dt = time.perf_counter() - t0
+  if args.dump_outputs:
+    bases, quals = opost.to_ascii(y, q)
+    dump_outputs(args.dump_outputs, bases=bases, quals=quals)
   value = sample * args.steps / dt
   desc = dict(value=value, unit=UNIT, cores=cores, kind="port",
               sample="%d synthetic windows per step (the full batch), torch-CPU fp32 oracle incl. argmax / QV" % sample)
@@ -222,7 +245,12 @@ def main():
   ap.add_argument("--nccl-scatter", action="store_true",
                   help="N > 1: also time the step fed by ONE reader rank over NCCL (BASELINE configs[3]; secondary record, "
                        "profiles/r02_bench_{2,4,8}gpu.json were produced with it)")
+  ap.add_argument("--dump-outputs", metavar="DIR",
+                  help="write the base and quality characters of the last timed step as DIR/bases.npy and DIR/quals.npy "
+                       "(float32 [batch, window]; rank 0's shard when N > 1; a fixed sample of windows above 64 MB)")
   args = ap.parse_args()
+  if args.steps < 1:
+    ap.error("--steps must be at least 1")
   args.warmup = max(args.warmup, 3)
 
   rank = int(os.environ.get("RANK", "0"))
@@ -383,6 +411,12 @@ def main():
   for _ in range(TRIALS):       # resident and host-buffer trials alternate, so both see the same thermal / power state
     res_trials.append(trial(run_resident_pipelined))                             # per-kernel events OFF
     e2e_trials.append(trial(run_e2e_pipelined))
+  if args.dump_outputs and rank == 0:
+    # the host-buffer trials write elsewhere, so the device outputs still hold the last step of the last `value` trial
+    bases, quals = np.empty((B, L), np.uint8), np.empty((B, L), np.uint8)
+    model.memcpy_d2h(bases, dev_bases)
+    model.memcpy_d2h(quals, dev_quals)
+    dump_outputs(args.dump_outputs, bases=bases, quals=quals)
   res_f32 = [trial(lambda n: run_resident_pipelined(n, packed=False)) for _ in range(3)]
   run_e2e_pipelined(3, packed=False)
   f32_trials = [trial(lambda n: run_e2e_pipelined(n, packed=False)) for _ in range(3)]

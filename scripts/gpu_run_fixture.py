@@ -1,4 +1,4 @@
-"""`deepconsensus_b200.run` on the reference's BAM fixtures (10 ZMWs, 1 593 windows), seeded weights: stage times."""
+"""`deepconsensus_b200.run` on the reference's BAM fixtures (7 of its 10 ZMWs, 958 windows), seeded weights: stage times."""
 import json, os, shutil, sys, tempfile, time
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from deepconsensus_b200 import run as run_lib

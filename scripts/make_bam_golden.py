@@ -3,9 +3,9 @@
 deepconsensus/testdata/human_1m/tf_examples/inference/inference.tfrecord.gz holds the 1 593 examples the reference's
 `deepconsensus preprocess` (v1.2.0, ins_trim=5: see tf_examples/summary/summary.inference.json) wrote from
 testdata/human_1m/{subreads_to_ccs,ccs}.bam.  This script reduces every example to (name, window_pos, num_passes,
-sha1 of the float32 rows, sha1 of the CCS base qualities) -> tests/golden/human_1m/inference_digest.json; byte copies of
-the two BAMs sit next to it.  tests/test_bam_prep.py rebuilds the windows from the BAMs with csrc/bam_prep.cpp and
-requires the same digest, window for window.  Run here (needs /root/reference); output is committed.
+sha1 of the float32 rows, sha1 of the CCS base qualities) -> tests/golden/human_1m/inference_digest.json; ccs.bam and
+7 of the 10 ZMWs of subreads_to_ccs.bam (scripts/make_bam_subset.py) sit next to it.  tests/test_bam_prep.py rebuilds
+the windows of those ZMWs with csrc/bam_prep.cpp and requires their digest entries, window for window.  Run here (needs /root/reference); output is committed.
 """
 import hashlib
 import importlib.util

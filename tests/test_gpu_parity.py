@@ -365,10 +365,11 @@ def test_device_post_model_stage_equals_reference_flow(engine_mod, golden_dir, c
 
 
 def test_run_from_bam_fixtures_end_to_end(engine_mod, golden_dir, tmp_path):
-  """BASELINE configs[0] (plumbing): `deepconsensus run` on the reference's own BAM fixtures (testdata/human_1m, 10 ZMWs,
-  1 593 windows) -- BAM -> features (C++) -> skip / model / fill / stitch (CUDA) -> FASTQ and BAM.  The fixture model
-  directory ships without its data shard, so the variables are seeded; the check is that the whole native flow gives
-  the records the reference flow on per-window Python objects gives, and that FASTQ and BAM outputs agree."""
+  """BASELINE configs[0] (plumbing): `deepconsensus run` on the reference's own BAM fixtures (testdata/human_1m; the
+  stored subread BAM keeps 7 of its 10 ZMWs, 958 windows) -- BAM -> features (C++) -> skip / model / fill / stitch
+  (CUDA) -> FASTQ and BAM.  The fixture model directory ships without its data shard, so the variables are seeded; the
+  check is that the whole native flow gives the records the reference flow on per-window Python objects gives, and that
+  FASTQ and BAM outputs agree."""
   import gzip, itertools, shutil
   from deepconsensus_b200 import inference, preprocess, run as run_lib, stitch_utils
   d = os.path.join(golden_dir, "human_1m")
@@ -380,7 +381,7 @@ def test_run_from_bam_fixtures_end_to_end(engine_mod, golden_dir, tmp_path):
   cnt = run_lib.run(output=fq, **args)
   bam = str(tmp_path / "out.bam")
   cnt2 = run_lib.run(output=bam, **args)
-  assert cnt.__dict__ == cnt2.__dict__ and cnt.success + cnt.failed_quality_filter + cnt.empty_sequence + cnt.only_gaps == 10
+  assert cnt.__dict__ == cnt2.__dict__ and cnt.success + cnt.failed_quality_filter + cnt.empty_sequence + cnt.only_gaps == 7
   got = open(fq).read()
   # reference flow from per-window objects
   p = params_lib.read_params_from_json(str(ck / "checkpoint-1"))
@@ -403,7 +404,7 @@ def test_run_from_bam_fixtures_end_to_end(engine_mod, golden_dir, tmp_path):
       want.append(rec)
   # the run processes ZMWs in batches of 4 in file order and sorts within a batch; compare as sets of records
   assert sorted(got.split("@")[1:]) == sorted("".join(want).split("@")[1:])
-  assert cnt.__dict__ == want_cnt.__dict__ and cnt.success >= 8
+  assert cnt.__dict__ == want_cnt.__dict__ and cnt.success >= 5
   # BAM output: same names / sequences / qualities as the FASTQ
   raw = open(bam, "rb").read()
   plain, pos = b"", 0
