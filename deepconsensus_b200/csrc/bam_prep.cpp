@@ -9,7 +9,8 @@
 //                                                     pw / ip reversed for reverse-strand alignments
 //   construct_ccs_read           pre_lib.py:966-998
 //   space_out_subreads           pre_lib.py:1242-1276 columns opened in every read wherever any read has an insertion
-//   DcExample.iter_examples /    pre_lib.py:625-744   windows of max_length columns, padding, the [R, L] feature rows --
+//   DcExample.iter_examples /    pre_lib.py:625-744   windows of max_length columns (or of the CCS record's `wl` widths),
+//                                                     padding, the [R, L] feature rows --
 //   extract_features                                  written as float32 rows AND as packed rows (dcb_pack_rows' format)
 //   unaligned BAM writer         quick_inference.py:740-760,892-897  (ec, np, rq, RG, zm tags; the CCS BAM's header)
 //
@@ -449,6 +450,7 @@ struct ZmwState {
   int has_ec = 0, has_np = 0, has_rq = 0, has_rg = 0;
   int32_t np_passes = 0, n_subreads = 0, ccs_length = 0;
   std::vector<int32_t> win_start; // column of every emitted window
+  std::vector<int32_t> win_width; // its spaced width (max_length for fixed-width windows)
   int rc = DCB_OK;                // error of the processing step (message in `error`)
   std::string error;
 };
@@ -459,7 +461,36 @@ struct ZmwJob {
   std::string name;
 };
 
-struct PrepCfg { int P = 0, L = 0, bq = 0, ins_trim = 0, R = 0; dcb::PackedLayout pl{}; };
+struct PrepCfg { int P = 0, L = 0, bq = 0, ins_trim = 0, R = 0, smart = 0; dcb::PackedLayout pl{}; };
+
+// DcExample.calculate_windows with window_widths (pre_lib.py:625-650): the `wl` tag of the CCS record gives every
+// window's width in CCS bases; walking the spaced CCS row, window i ends once wl[i] non-gap columns are behind it.
+// The reference raises where the tag is missing (KeyError), where sum(wl) walks past the row (IndexError) and where the
+// spaced widths do not add up to ccs_width (assert); those cases are errors here too.
+int smart_window_widths(const BamRecord& c, const Read& ccs, int ccs_width, std::vector<int32_t>* widths) {
+  Tag t;
+  if (!c.find("wl", &t)) return pfail(DCB_ERR_INVALID, "%s: no wl tag (needed for CCS smart windows)", c.qname.c_str());
+  if (t.type != 'B' || !t.sub || !strchr("cCsSiI", t.sub))
+    return pfail(DCB_ERR_INVALID, "%s: the wl tag is not an integer array", c.qname.c_str());
+  const int64_t width = (int64_t)ccs.bases.size();
+  int64_t last = 0;
+  for (size_t i = 0; i < t.count; ++i) {
+    const int64_t want = (int64_t)BamRecord::element(t, i);
+    int64_t orig = 0, spaced = 0;
+    while (orig < want) {
+      if (last + spaced >= width)
+        return pfail(DCB_ERR_INVALID, "%s: the wl tag covers more than the CCS read's %zu bases", c.qname.c_str(), c.seq.size());
+      if (ccs.bases[last + spaced] != kGap) ++orig;
+      ++spaced;
+    }
+    widths->push_back((int32_t)spaced);
+    last += spaced;
+  }
+  if (last != ccs_width)
+    return pfail(DCB_ERR_INVALID, "%s: the wl tag's windows span %lld columns, the spaced CCS read %d", c.qname.c_str(),
+                 (long long)last, ccs_width);
+  return DCB_OK;
+}
 
 // CPU-heavy part, no I/O: expand_clip_indent per subread, construct_ccs_read, space_out_subreads, window list
 void process_zmw(const PrepCfg& cfg, ZmwJob* job, ZmwState* st) {
@@ -480,23 +511,52 @@ void process_zmw(const PrepCfg& cfg, ZmwJob* job, ZmwState* st) {
   st->has_rg = c.find("RG", &t) && t.type == 'Z'; if (st->has_rg) st->rg = reinterpret_cast<const char*>(t.p);
   st->ccs_length = (int32_t)c.seq.size();
   space_out(st->reads);
-  // DcExample.iter_examples (pre_lib.py:625-697), fixed-width windows
+  // DcExample.iter_examples (pre_lib.py:625-697): windows of max_length columns, or of the widths the wl tag gives
   const Read& ccs = st->reads.back();
   const int width = (int)ccs.bases.size();
   int ccs_width = width;
   while (ccs_width > 0 && (ccs.bases[ccs_width - 1] == ' ' || ccs.bases[ccs_width - 1] == '\t' || ccs.bases[ccs_width - 1] == '\n')) --ccs_width;
-  const int nwin = (ccs_width + cfg.L - 1) / cfg.L;
+  std::vector<int32_t> widths;
+  if (cfg.smart) {
+    if (smart_window_widths(c, ccs, ccs_width, &widths)) { st->rc = DCB_ERR_INVALID; st->error = g_prep_error; return; }
+  } else {
+    widths.assign((ccs_width + cfg.L - 1) / cfg.L, cfg.L);
+  }
   st->win_start.clear();
+  st->win_width.clear();
   int start = 0;
-  for (int w = 0; w < nwin; ++w) {
+  for (const int32_t ww : widths) {
     if (start > ccs_width) break;
     const int s0 = start;
-    start += cfg.L;
+    start += ww;
     bool any = false;
-    for (int i = s0; i < std::min(s0 + cfg.L, width); ++i) any |= ccs.ccs_idx[i] >= 0;
+    for (int i = s0; i < std::min(s0 + ww, width); ++i) any |= ccs.ccs_idx[i] >= 0;
     if (!any) continue;                                         // n_examples_no_ccs_idx
     st->win_start.push_back(s0);
+    st->win_width.push_back(ww);                                // overflow: ww > max_length
   }
+}
+
+// extract_features (pre_lib.py:704-744) of the columns [s, s + n) into float32 rows [R, Wo]; columns n..Wo-1 are padding
+void write_rows(const ZmwState& st, const PrepCfg& cf, int s, int n, int Wo, float* d) {
+  const int P = cf.P, R = cf.R;
+  const int keep = (int)std::min<size_t>(P, st.reads.size() - 1);
+  const Read& ccs = st.reads.back();
+  memset(d, 0, sizeof(float) * (size_t)R * Wo);
+  for (int k = 0; k < keep; ++k) {
+    const Read& r = st.reads[k];
+    for (int i = 0; i < n; ++i) {
+      d[(size_t)k * Wo + i] = encode_base(r.bases[s + i]);
+      d[(size_t)(P + k) * Wo + i] = (float)r.pw[s + i];
+      d[(size_t)(2 * P + k) * Wo + i] = (float)r.ip[s + i];
+    }
+    for (int i = 0; i < Wo; ++i) d[(size_t)(3 * P + k) * Wo + i] = (float)r.strand;   // repeated over the whole width
+  }
+  for (int i = 0; i < n; ++i) d[(size_t)4 * P * Wo + i] = encode_base(ccs.bases[s + i]);
+  if (cf.bq)
+    for (int i = 0; i < Wo; ++i) d[(size_t)(4 * P + 1) * Wo + i] = (i < n && ccs.bq_any) ? (float)ccs.bq[s + i] : -1.f;
+  for (int j = 0; j < 4; ++j)
+    for (int i = 0; i < Wo; ++i) d[(size_t)(R - 4 + j) * Wo + i] = st.reads[0].sn[j];
 }
 
 }  // namespace
@@ -650,6 +710,14 @@ int dcb_prep_set_threads(dcb_prep* p, int32_t n_threads) {
   return DCB_OK;
 }
 
+// Windows from the CCS record's `wl` tag instead of max_length columns (--use_ccs_smart_windows, pre_lib.py:1329-1331).
+int dcb_prep_set_smart_windows(dcb_prep* p, int32_t enable) {
+  if (!p) return pfail(DCB_ERR_INVALID, "dcb_prep_set_smart_windows: null handle");
+  if (p->started || p->next_seq) return pfail(DCB_ERR_STATE, "dcb_prep_set_smart_windows: the stream has already started");
+  p->cfg.smart = enable ? 1 : 0;
+  return DCB_OK;
+}
+
 void dcb_prep_close(dcb_prep* p) {
   if (!p) return;
   stop_threads(p);
@@ -702,7 +770,8 @@ int dcb_prep_next_zmw(dcb_prep* p, dcb_zmw_info* info) {
 
 // The windows of the current ZMW (DcExample.extract_features / to_features_dict, pre_lib.py:704-762).  Every output may
 // be NULL.  rows: float32 [n, R, L]; packed: [n, packed_window_bytes]; window_pos / num_passes: [n]; overflow: [n]
-// (always 0 with fixed-width windows); ccs_bq: int16 [n, L] (-1 at gaps and padding).
+// (always 0 with fixed-width windows); ccs_bq: int16 [n, L] (-1 at gaps and padding).  An overflow window (smart
+// windows wider than max_length) appears here with its first L columns; dcb_prep_get_overflow_windows has all of it.
 int dcb_prep_get_windows(dcb_prep* p, float* rows, uint8_t* packed, int32_t* window_pos, uint8_t* overflow,
                          int16_t* ccs_bq, int32_t* num_passes) {
   if (!p) return pfail(DCB_ERR_INVALID, "dcb_prep_get_windows: null handle");
@@ -715,26 +784,10 @@ int dcb_prep_get_windows(dcb_prep* p, float* rows, uint8_t* packed, int32_t* win
   const Read& ccs = st.reads.back();
   const int width = (int)ccs.bases.size();
   for (size_t w = 0; w < st.win_start.size(); ++w) {
-    const int s = st.win_start[w];
-    const int n = std::min(L, width - s);                      // columns present; the rest is padding
-    if (rows) {
-      float* d = rows + w * (size_t)R * L;
-      memset(d, 0, sizeof(float) * (size_t)R * L);
-      for (int k = 0; k < keep; ++k) {
-        const Read& r = st.reads[k];
-        for (int i = 0; i < n; ++i) {
-          d[(size_t)k * L + i] = encode_base(r.bases[s + i]);
-          d[(size_t)(P + k) * L + i] = (float)r.pw[s + i];
-          d[(size_t)(2 * P + k) * L + i] = (float)r.ip[s + i];
-        }
-        for (int i = 0; i < L; ++i) d[(size_t)(3 * P + k) * L + i] = (float)r.strand;   // repeated over the whole width
-      }
-      for (int i = 0; i < n; ++i) d[(size_t)4 * P * L + i] = encode_base(ccs.bases[s + i]);
-      if (cf.bq)
-        for (int i = 0; i < L; ++i) d[(size_t)(4 * P + 1) * L + i] = (i < n && ccs.bq_any) ? (float)ccs.bq[s + i] : -1.f;
-      for (int j = 0; j < 4; ++j)
-        for (int i = 0; i < L; ++i) d[(size_t)(R - 4 + j) * L + i] = st.reads[0].sn[j];
-    }
+    const int s = st.win_start[w], ww = st.win_width[w];
+    const int nw = std::min(ww, width - s);                   // columns of the window
+    const int n = std::min(L, nw);                             // of those, the ones in the first L; the rest is padding
+    if (rows) write_rows(st, cf, s, n, L, rows + w * (size_t)R * L);
     if (packed) {
       uint8_t* o = packed + w * (size_t)cf.pl.stride;
       memset(o, 0, cf.pl.stride);
@@ -754,16 +807,45 @@ int dcb_prep_get_windows(dcb_prep* p, float* rows, uint8_t* packed, int32_t* win
     if (window_pos) {
       int32_t mn = 0;
       bool found = false;
-      for (int i = 0; i < n; ++i) {
+      for (int i = 0; i < nw; ++i) {
         const int32_t v = ccs.ccs_idx[s + i];
         if (v >= 0 && (!found || v < mn)) { mn = v; found = true; }
       }
       window_pos[w] = mn;                                       // ccs_bounds.start
     }
-    if (overflow) overflow[w] = 0;
+    if (overflow) overflow[w] = ww > L;
     if (num_passes) num_passes[w] = keep;
     if (ccs_bq)
       for (int i = 0; i < L; ++i) ccs_bq[w * (size_t)L + i] = (int16_t)((i < n && ccs.bq_any) ? ccs.bq[s + i] : -1);
+  }
+  return DCB_OK;
+}
+
+int dcb_prep_get_window_widths(dcb_prep* p, int32_t* widths) {
+  if (!p || !widths) return pfail(DCB_ERR_INVALID, "dcb_prep_get_window_widths: null argument");
+  if (p->cur.reads.empty()) return pfail(DCB_ERR_STATE, "dcb_prep_get_window_widths: no ZMW loaded");
+  std::copy(p->cur.win_width.begin(), p->cur.win_width.end(), widths);
+  return DCB_OK;
+}
+
+// The overflow windows of the current ZMW in full, ragged: window after window, W columns each.
+int dcb_prep_get_overflow_windows(dcb_prep* p, float* rows, uint8_t* ccs_ids, int16_t* ccs_bq) {
+  if (!p) return pfail(DCB_ERR_INVALID, "dcb_prep_get_overflow_windows: null handle");
+  const ZmwState& st = p->cur;
+  if (st.reads.empty()) return pfail(DCB_ERR_STATE, "dcb_prep_get_overflow_windows: no ZMW loaded");
+  const PrepCfg& cf = p->cfg;
+  const Read& ccs = st.reads.back();
+  size_t off = 0;
+  for (size_t w = 0; w < st.win_start.size(); ++w) {
+    const int s = st.win_start[w], ww = st.win_width[w];
+    if (ww <= cf.L) continue;
+    const int n = std::min(ww, (int)ccs.bases.size() - s);
+    if (rows) write_rows(st, cf, s, n, ww, rows + off * cf.R);
+    for (int i = 0; i < ww; ++i) {
+      if (ccs_ids) ccs_ids[off + i] = (uint8_t)(i < n ? encode_base(ccs.bases[s + i]) : 0);
+      if (ccs_bq) ccs_bq[off + i] = (int16_t)((i < n && ccs.bq_any) ? ccs.bq[s + i] : -1);
+    }
+    off += ww;
   }
   return DCB_OK;
 }

@@ -115,6 +115,7 @@ struct dcb_engine {
   // stitch scratch (grown on demand)
   uint8_t *d_st_in = nullptr, *d_st_out = nullptr;   // [2][cap] each: bases|quals, seq|qual
   int32_t *d_st_start = nullptr, *d_st_len = nullptr;
+  int64_t* d_st_off = nullptr;                        // byte offset of every read (n_zmw + 1)
   size_t st_cap = 0, st_zcap = 0;
   // post-model stage scratch (dcb_stitch_fastq / dcb_skip_mask / dcb_fill_skipped), grown on demand
   double* d_p10 = nullptr;           // 10^(-q/10), q = 0..255 (host libm pow, as NumPy)
@@ -338,6 +339,7 @@ void dcb_destroy(dcb_engine* e) {
   if (e->d_st_out) cudaFree(e->d_st_out);
   if (e->d_st_start) cudaFree(e->d_st_start);
   if (e->d_st_len) cudaFree(e->d_st_len);
+  if (e->d_st_off) cudaFree(e->d_st_off);
   for (dcb_engine::Scratch* sc : {&e->sc_pos, &e->sc_names, &e->sc_nameoff, &e->sc_outcome, &e->sc_avg, &e->sc_recoff,
                                   &e->sc_fastq, &e->sc_bq, &e->sc_mask, &e->sc_ids, &e->sc_dst, &e->sc_tmpb, &e->sc_tmpq})
     if (sc->p) cudaFree(sc->p);
@@ -1260,6 +1262,12 @@ int dcb_debug_residual(dcb_engine* e, int32_t stage, float* out, int64_t out_ele
   return DCB_OK;
 }
 
+namespace {
+int stitch_spans(dcb_engine* e, const uint8_t* bases, const uint8_t* quals, size_t nbytes, const int64_t* read_off,
+                 const int32_t* zmw_start, int32_t n_zmw, uint32_t flags, uint8_t* seq_out, uint8_t* qual_out,
+                 int32_t* len_out);
+}  // namespace
+
 int dcb_stitch(dcb_engine* e, const uint8_t* bases, const uint8_t* quals, int32_t n_windows, int32_t L,
                const int32_t* zmw_start, int32_t n_zmw, uint32_t flags,
                uint8_t* seq_out, uint8_t* qual_out, int32_t* len_out) {
@@ -1270,8 +1278,21 @@ int dcb_stitch(dcb_engine* e, const uint8_t* bases, const uint8_t* quals, int32_
   if (zmw_start[0] < 0 || zmw_start[n_zmw] > n_windows) return fail(e, DCB_ERR_INVALID, "dcb_stitch: zmw_start outside [0, n_windows]");
   for (int z = 0; z < n_zmw; ++z)
     if (zmw_start[z + 1] < zmw_start[z]) return fail(e, DCB_ERR_INVALID, "dcb_stitch: zmw_start must be non-decreasing");
+  std::vector<int64_t> read_off((size_t)n_zmw + 1);
+  for (int z = 0; z <= n_zmw; ++z) read_off[z] = (int64_t)zmw_start[z] * L;
+  return stitch_spans(e, bases, quals, (size_t)n_windows * L, read_off.data(), zmw_start, n_zmw, flags, seq_out, qual_out,
+                      len_out);
+}
+
+namespace {
+// dcb_stitch on byte spans: read z is bytes [read_off[z], read_off[z + 1]) of bases / quals (nbytes in all; host int64
+// offsets) and is written at the same offsets of seq_out / qual_out.  zmw_start is left in d_st_start, read_off in d_st_off.
+int stitch_spans(dcb_engine* e, const uint8_t* bases, const uint8_t* quals, size_t nbytes, const int64_t* read_off,
+                 const int32_t* zmw_start, int32_t n_zmw, uint32_t flags, uint8_t* seq_out, uint8_t* qual_out,
+                 int32_t* len_out) {
+  for (int z = 0; z < n_zmw; ++z)
+    if (read_off[z + 1] - read_off[z] > INT32_MAX) return fail(e, DCB_ERR_INVALID, "dcb_stitch: read %d spans 2^31 bytes or more", z);
   CU(e, cudaSetDevice(e->cfg.device));
-  const size_t nbytes = (size_t)n_windows * L;
   const bool in_dev = flags & DCB_ROWS_ON_DEVICE, out_dev = flags & DCB_OUT_ON_DEVICE;
   cudaStream_t st = e->stream;
   if (nbytes > e->st_cap) {
@@ -1288,10 +1309,13 @@ int dcb_stitch(dcb_engine* e, const uint8_t* bases, const uint8_t* quals, int32_
     CU(e, cudaStreamSynchronize(st));
     if (e->d_st_start) cudaFree(e->d_st_start);
     if (e->d_st_len) cudaFree(e->d_st_len);
+    if (e->d_st_off) cudaFree(e->d_st_off);
     e->d_st_start = e->d_st_len = nullptr;
+    e->d_st_off = nullptr;
     e->st_zcap = 0;
     CU(e, cudaMalloc(reinterpret_cast<void**>(&e->d_st_start), ((size_t)n_zmw + 1) * sizeof(int32_t)));
     CU(e, cudaMalloc(reinterpret_cast<void**>(&e->d_st_len), ((size_t)n_zmw + 1) * sizeof(int32_t)));
+    CU(e, cudaMalloc(reinterpret_cast<void**>(&e->d_st_off), ((size_t)n_zmw + 1) * sizeof(int64_t)));
     e->st_zcap = (size_t)n_zmw + 1;
   }
   const uint8_t *db = bases, *dq = quals;
@@ -1301,10 +1325,11 @@ int dcb_stitch(dcb_engine* e, const uint8_t* bases, const uint8_t* quals, int32_
     db = e->d_st_in; dq = e->d_st_in + e->st_cap;
   }
   CU(e, cudaMemcpyAsync(e->d_st_start, zmw_start, ((size_t)n_zmw + 1) * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+  CU(e, cudaMemcpyAsync(e->d_st_off, read_off, ((size_t)n_zmw + 1) * sizeof(int64_t), cudaMemcpyHostToDevice, st));
   uint8_t* ds = out_dev ? seq_out : e->d_st_out;
   uint8_t* dqo = out_dev ? qual_out : e->d_st_out + e->st_cap;
   int32_t* dl = out_dev ? len_out : e->d_st_len;
-  launch_stitch(db, dq, L, e->d_st_start, n_zmw, ds, dqo, dl, st);
+  launch_stitch(db, dq, e->d_st_off, n_zmw, ds, dqo, dl, st);
   if (!out_dev) {
     CU(e, cudaMemcpyAsync(seq_out, ds, nbytes, cudaMemcpyDeviceToHost, st));
     CU(e, cudaMemcpyAsync(qual_out, dqo, nbytes, cudaMemcpyDeviceToHost, st));
@@ -1315,7 +1340,6 @@ int dcb_stitch(dcb_engine* e, const uint8_t* bases, const uint8_t* quals, int32_
   return DCB_OK;
 }
 
-namespace {
 // grow-on-demand device scratch; contents are not preserved
 int ensure(dcb_engine* e, dcb_engine::Scratch& sc, size_t bytes) {
   if (bytes <= sc.cap) return DCB_OK;
@@ -1333,15 +1357,36 @@ int dcb_stitch_fastq(dcb_engine* e, const uint8_t* bases, const uint8_t* quals, 
                      const int32_t* name_off, double min_quality, int32_t min_length, uint32_t flags, uint8_t* fastq_out,
                      int64_t fastq_cap, int64_t* rec_off, int32_t* outcome, double* avg_q) {
   if (!e) return DCB_ERR_INVALID;
+  if (n_windows < 0 || L <= 0) return fail(e, DCB_ERR_INVALID, "dcb_stitch_fastq: negative size");
+  std::vector<int64_t> window_off((size_t)n_windows + 1);
+  for (int w = 0; w <= n_windows; ++w) window_off[w] = (int64_t)w * L;
+  return dcb_stitch_fastq_ragged(e, bases, quals, n_windows, window_off.data(), L, zmw_start, n_zmw, window_pos, names,
+                                 name_off, min_quality, min_length, flags, fastq_out, fastq_cap, rec_off, outcome, avg_q);
+}
+
+int dcb_stitch_fastq_ragged(dcb_engine* e, const uint8_t* bases, const uint8_t* quals, int32_t n_windows,
+                            const int64_t* window_off, int32_t L, const int32_t* zmw_start, int32_t n_zmw,
+                            const int32_t* window_pos, const uint8_t* names, const int32_t* name_off, double min_quality,
+                            int32_t min_length, uint32_t flags, uint8_t* fastq_out, int64_t fastq_cap, int64_t* rec_off,
+                            int32_t* outcome, double* avg_q) {
+  if (!e) return DCB_ERR_INVALID;
   if (n_windows < 0 || L <= 0 || n_zmw < 0 || fastq_cap < 0) return fail(e, DCB_ERR_INVALID, "dcb_stitch_fastq: negative size");
   if (!rec_off) return fail(e, DCB_ERR_INVALID, "dcb_stitch_fastq: null pointer");
   if (n_zmw == 0) { rec_off[0] = 0; return DCB_OK; }
-  if (!bases || !quals || !zmw_start || !window_pos || !names || !name_off || !fastq_out || !outcome || !avg_q)
+  if (!bases || !quals || !window_off || !zmw_start || !window_pos || !names || !name_off || !fastq_out || !outcome || !avg_q)
     return fail(e, DCB_ERR_INVALID, "dcb_stitch_fastq: null pointer");
   if (name_off[0] != 0) return fail(e, DCB_ERR_INVALID, "dcb_stitch_fastq: name_off[0] must be 0");
   for (int z = 0; z < n_zmw; ++z)
     if (name_off[z + 1] < name_off[z]) return fail(e, DCB_ERR_INVALID, "dcb_stitch_fastq: name_off must be non-decreasing");
-  const size_t nbytes = (size_t)n_windows * L;
+  if (zmw_start[0] < 0 || zmw_start[n_zmw] > n_windows) return fail(e, DCB_ERR_INVALID, "dcb_stitch_fastq: zmw_start outside [0, n_windows]");
+  for (int z = 0; z < n_zmw; ++z)
+    if (zmw_start[z + 1] < zmw_start[z]) return fail(e, DCB_ERR_INVALID, "dcb_stitch_fastq: zmw_start must be non-decreasing");
+  if (window_off[0] < 0) return fail(e, DCB_ERR_INVALID, "dcb_stitch_fastq: negative window offset");
+  for (int w = 0; w < n_windows; ++w)
+    if (window_off[w + 1] < window_off[w]) return fail(e, DCB_ERR_INVALID, "dcb_stitch_fastq: window_off must be non-decreasing");
+  std::vector<int64_t> read_off((size_t)n_zmw + 1);
+  for (int z = 0; z <= n_zmw; ++z) read_off[z] = window_off[zmw_start[z]];
+  const size_t nbytes = (size_t)window_off[n_windows];
   // stage 1: concatenation + gap compaction (dcb_stitch), results stay on the device
   CU(e, cudaSetDevice(e->cfg.device));
   cudaStream_t st = e->stream;
@@ -1353,31 +1398,35 @@ int dcb_stitch_fastq(dcb_engine* e, const uint8_t* bases, const uint8_t* quals, 
   uint8_t* d_seq = static_cast<uint8_t*>(e->sc_tmpb.p);
   uint8_t* d_qual = static_cast<uint8_t*>(e->sc_tmpq.p);
   int32_t* d_len = static_cast<int32_t*>(e->sc_dst.p);
-  if (n_windows > 0) {
-    rc = dcb_stitch(e, bases, quals, n_windows, L, zmw_start, n_zmw, (flags & DCB_ROWS_ON_DEVICE) | DCB_OUT_ON_DEVICE, d_seq, d_qual, d_len);
+  if (nbytes > 0) {
+    rc = stitch_spans(e, bases, quals, nbytes, read_off.data(), zmw_start, n_zmw, (flags & DCB_ROWS_ON_DEVICE) | DCB_OUT_ON_DEVICE,
+                      d_seq, d_qual, d_len);
     if (rc) return rc;
   } else {
     CU(e, cudaMemsetAsync(d_len, 0, ((size_t)n_zmw + 1) * sizeof(int32_t), st));
   }
   const size_t names_bytes = (size_t)name_off[n_zmw];
   const size_t cap = (size_t)fastq_cap;
-  if ((rc = ensure(e, e->sc_pos, (nbytes ? (size_t)n_windows : 1) * sizeof(int32_t))) ||
+  if ((rc = ensure(e, e->sc_pos, (n_windows ? (size_t)n_windows : 1) * sizeof(int32_t))) ||
       (rc = ensure(e, e->sc_names, names_bytes ? names_bytes : 1)) ||
       (rc = ensure(e, e->sc_nameoff, ((size_t)n_zmw + 1) * sizeof(int32_t))) ||
       (rc = ensure(e, e->sc_outcome, (size_t)n_zmw * sizeof(int32_t))) || (rc = ensure(e, e->sc_avg, (size_t)n_zmw * sizeof(double))) ||
       (rc = ensure(e, e->sc_recoff, ((size_t)n_zmw + 1) * sizeof(int64_t))) || (rc = ensure(e, e->sc_fastq, cap ? cap : 1)))
     return rc;
-  // dcb_stitch left zmw_start in its own scratch (d_st_start)
-  if (n_windows == 0) {
+  // stitch_spans left zmw_start / read_off in its own scratch (d_st_start / d_st_off)
+  if (nbytes == 0) {
     if ((size_t)n_zmw + 1 > e->st_zcap) {
       if (e->d_st_start) cudaFree(e->d_st_start);
       if (e->d_st_len) cudaFree(e->d_st_len);
-      e->d_st_start = e->d_st_len = nullptr; e->st_zcap = 0;
+      if (e->d_st_off) cudaFree(e->d_st_off);
+      e->d_st_start = e->d_st_len = nullptr; e->d_st_off = nullptr; e->st_zcap = 0;
       CU(e, cudaMalloc(reinterpret_cast<void**>(&e->d_st_start), ((size_t)n_zmw + 1) * sizeof(int32_t)));
       CU(e, cudaMalloc(reinterpret_cast<void**>(&e->d_st_len), ((size_t)n_zmw + 1) * sizeof(int32_t)));
+      CU(e, cudaMalloc(reinterpret_cast<void**>(&e->d_st_off), ((size_t)n_zmw + 1) * sizeof(int64_t)));
       e->st_zcap = (size_t)n_zmw + 1;
     }
     CU(e, cudaMemcpyAsync(e->d_st_start, zmw_start, ((size_t)n_zmw + 1) * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+    CU(e, cudaMemcpyAsync(e->d_st_off, read_off.data(), ((size_t)n_zmw + 1) * sizeof(int64_t), cudaMemcpyHostToDevice, st));
   }
   if (n_windows > 0) CU(e, cudaMemcpyAsync(e->sc_pos.p, window_pos, (size_t)n_windows * sizeof(int32_t), cudaMemcpyHostToDevice, st));
   if (names_bytes) CU(e, cudaMemcpyAsync(e->sc_names.p, names, names_bytes, cudaMemcpyHostToDevice, st));
@@ -1385,9 +1434,9 @@ int dcb_stitch_fastq(dcb_engine* e, const uint8_t* bases, const uint8_t* quals, 
   int32_t* d_out = static_cast<int32_t*>(e->sc_outcome.p);
   double* d_avg = static_cast<double*>(e->sc_avg.p);
   int64_t* d_rec = static_cast<int64_t*>(e->sc_recoff.p);
-  launch_read_outcome(d_qual, d_len, e->d_st_start, static_cast<const int32_t*>(e->sc_pos.p), L, n_zmw, e->d_p10, min_quality,
-                      min_length, d_out, d_avg, st);
-  launch_fastq(d_seq, d_qual, d_len, e->d_st_start, L, n_zmw, d_out, static_cast<const uint8_t*>(e->sc_names.p),
+  launch_read_outcome(d_qual, d_len, e->d_st_off, e->d_st_start, static_cast<const int32_t*>(e->sc_pos.p), L, n_zmw, e->d_p10,
+                      min_quality, min_length, d_out, d_avg, st);
+  launch_fastq(d_seq, d_qual, d_len, e->d_st_off, n_zmw, d_out, static_cast<const uint8_t*>(e->sc_names.p),
                static_cast<const int32_t*>(e->sc_nameoff.p), d_rec, static_cast<uint8_t*>(e->sc_fastq.p), fastq_cap, st);
   CU(e, cudaMemcpyAsync(rec_off, d_rec, ((size_t)n_zmw + 1) * sizeof(int64_t), cudaMemcpyDeviceToHost, st));
   CU(e, cudaMemcpyAsync(outcome, d_out, (size_t)n_zmw * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
@@ -1431,26 +1480,46 @@ int dcb_fill_skipped(dcb_engine* e, const uint8_t* ccs_ids, const int16_t* ccs_b
   if (!ccs_ids || !ccs_bq || !dst_window || !bases || !quals) return fail(e, DCB_ERR_INVALID, "dcb_fill_skipped: null pointer");
   for (int j = 0; j < k; ++j)
     if (dst_window[j] < 0) return fail(e, DCB_ERR_INVALID, "dcb_fill_skipped: negative destination window");
+  std::vector<int64_t> src_off((size_t)k + 1), dst_off((size_t)k);
+  for (int j = 0; j <= k; ++j) src_off[j] = (int64_t)j * L;
+  for (int j = 0; j < k; ++j) dst_off[j] = (int64_t)dst_window[j] * L;
+  return dcb_fill_skipped_ragged(e, ccs_ids, ccs_bq, src_off.data(), dst_off.data(), k, calibration_enabled,
+                                 calibration_threshold, calibration_w, calibration_b, flags, bases, quals);
+}
+
+int dcb_fill_skipped_ragged(dcb_engine* e, const uint8_t* ccs_ids, const int16_t* ccs_bq, const int64_t* src_off,
+                            const int64_t* dst_off, int32_t k, int32_t calibration_enabled, double calibration_threshold,
+                            double calibration_w, double calibration_b, uint32_t flags, uint8_t* bases, uint8_t* quals) {
+  if (!e) return DCB_ERR_INVALID;
+  if (k < 0) return fail(e, DCB_ERR_INVALID, "dcb_fill_skipped: negative size");
+  if (k == 0) return DCB_OK;
+  if (!ccs_ids || !ccs_bq || !src_off || !dst_off || !bases || !quals) return fail(e, DCB_ERR_INVALID, "dcb_fill_skipped: null pointer");
+  if (src_off[0] != 0) return fail(e, DCB_ERR_INVALID, "dcb_fill_skipped: src_off[0] must be 0");
+  for (int j = 0; j < k; ++j)
+    if (src_off[j + 1] < src_off[j] || dst_off[j] < 0)
+      return fail(e, DCB_ERR_INVALID, "dcb_fill_skipped: src_off must be non-decreasing, dst_off non-negative");
   CU(e, cudaSetDevice(e->cfg.device));
   cudaStream_t st = e->stream;
-  const size_t n = (size_t)k * L;
+  const size_t n = (size_t)src_off[k];
   const bool out_dev = flags & DCB_OUT_ON_DEVICE;
   int rc;
-  if ((rc = ensure(e, e->sc_ids, n)) || (rc = ensure(e, e->sc_bq, n * sizeof(int16_t))) ||
-      (rc = ensure(e, e->sc_dst, ((size_t)k + 1) * sizeof(int32_t))) || (rc = ensure(e, e->sc_mask, sizeof(int))))
+  if ((rc = ensure(e, e->sc_ids, n ? n : 1)) || (rc = ensure(e, e->sc_bq, (n ? n : 1) * sizeof(int16_t))) ||
+      (rc = ensure(e, e->sc_dst, (2 * (size_t)k + 1) * sizeof(int64_t))) || (rc = ensure(e, e->sc_mask, sizeof(int))))
     return rc;
-  if (!out_dev && ((rc = ensure(e, e->sc_tmpb, n)) || (rc = ensure(e, e->sc_tmpq, n)))) return rc;
-  std::vector<int32_t> dst(dst_window, dst_window + k);
-  if (!out_dev) for (int j = 0; j < k; ++j) dst[j] = j;      // dense temporary, scattered on the host below
+  if (!out_dev && ((rc = ensure(e, e->sc_tmpb, n ? n : 1)) || (rc = ensure(e, e->sc_tmpq, n ? n : 1)))) return rc;
+  int64_t* d_src = static_cast<int64_t*>(e->sc_dst.p);
+  int64_t* d_dst = d_src + k + 1;
   CU(e, cudaMemcpyAsync(e->sc_ids.p, ccs_ids, n, cudaMemcpyHostToDevice, st));
   CU(e, cudaMemcpyAsync(e->sc_bq.p, ccs_bq, n * sizeof(int16_t), cudaMemcpyHostToDevice, st));
-  CU(e, cudaMemcpyAsync(e->sc_dst.p, dst.data(), (size_t)k * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+  CU(e, cudaMemcpyAsync(d_src, src_off, ((size_t)k + 1) * sizeof(int64_t), cudaMemcpyHostToDevice, st));
+  // host outputs: a dense temporary laid out like the source, scattered on the host below
+  CU(e, cudaMemcpyAsync(d_dst, out_dev ? dst_off : src_off, (size_t)k * sizeof(int64_t), cudaMemcpyHostToDevice, st));
   CU(e, cudaMemsetAsync(e->sc_mask.p, 0, sizeof(int), st));
   uint8_t* db = out_dev ? bases : static_cast<uint8_t*>(e->sc_tmpb.p);
   uint8_t* dq = out_dev ? quals : static_cast<uint8_t*>(e->sc_tmpq.p);
-  launch_fill_skipped(static_cast<const uint8_t*>(e->sc_ids.p), static_cast<const int16_t*>(e->sc_bq.p),
-                      static_cast<const int32_t*>(e->sc_dst.p), k, L, calibration_enabled, calibration_threshold,
-                      calibration_w, calibration_b, e->cfg.max_base_quality, db, dq, static_cast<int*>(e->sc_mask.p), st);
+  launch_fill_skipped(static_cast<const uint8_t*>(e->sc_ids.p), static_cast<const int16_t*>(e->sc_bq.p), d_src, d_dst, k,
+                      calibration_enabled, calibration_threshold, calibration_w, calibration_b, e->cfg.max_base_quality,
+                      db, dq, static_cast<int*>(e->sc_mask.p), st);
   int status = 0;
   CU(e, cudaMemcpyAsync(&status, e->sc_mask.p, sizeof(int), cudaMemcpyDeviceToHost, st));
   if (!out_dev) {
@@ -1459,8 +1528,8 @@ int dcb_fill_skipped(dcb_engine* e, const uint8_t* ccs_ids, const int16_t* ccs_b
     CU(e, cudaMemcpyAsync(hq.data(), dq, n, cudaMemcpyDeviceToHost, st));
     CU(e, cudaStreamSynchronize(st));
     for (int j = 0; j < k; ++j) {
-      memcpy(bases + (size_t)dst_window[j] * L, hb.data() + (size_t)j * L, L);
-      memcpy(quals + (size_t)dst_window[j] * L, hq.data() + (size_t)j * L, L);
+      memcpy(bases + dst_off[j], hb.data() + src_off[j], (size_t)(src_off[j + 1] - src_off[j]));
+      memcpy(quals + dst_off[j], hq.data() + src_off[j], (size_t)(src_off[j + 1] - src_off[j]));
     }
   } else {
     CU(e, cudaStreamSynchronize(st));

@@ -3087,19 +3087,20 @@ int read_ffn_trace(unsigned long long* out, int n) {
 // =====================================================================================
 // stitch: per-read concatenation of windows + gap compaction (stitch_utils.py:51-98)
 // =====================================================================================
-// One CTA per read (ZMW).  Its windows are contiguous in the batch, so the read's input is one span of
-// (w1 - w0) * L bytes in `bases` / `quals`; the gap character ' ' and the quality character under it are dropped
-// (order preserving: ballot-free block prefix sum over 1024-character tiles) and the compacted read is written at the
-// same offset of seq_out / qual_out.  Integer / byte work only: bit-exact against the reference's string loops.
+// One CTA per read (ZMW).  Its windows are contiguous in the batch, so the read's input is one span of bytes
+// [read_off[z], read_off[z + 1]) in `bases` / `quals` (windows of max_length bytes, or of their own width when CCS smart
+// windows overflow); the gap character ' ' and the quality character under it are dropped (order preserving:
+// ballot-free block prefix sum over 1024-character tiles) and the compacted read is written at the same offset of
+// seq_out / qual_out.  Offsets are int64 (a batch may exceed 2 GiB of window bytes); one read stays below 2^31 bytes.  Integer / byte work only: bit-exact against the reference's string loops.
 __global__ void __launch_bounds__(256)
-stitch_kernel(const uint8_t* __restrict__ bases, const uint8_t* __restrict__ quals, int L,
-              const int32_t* __restrict__ zmw_start, uint8_t* __restrict__ seq_out, uint8_t* __restrict__ qual_out,
+stitch_kernel(const uint8_t* __restrict__ bases, const uint8_t* __restrict__ quals,
+              const int64_t* __restrict__ read_off, uint8_t* __restrict__ seq_out, uint8_t* __restrict__ qual_out,
               int32_t* __restrict__ len_out) {
   __shared__ int s_warp[8];
   __shared__ int s_total;
   const int z = blockIdx.x;
-  const size_t off = (size_t)zmw_start[z] * L;
-  const int n = (zmw_start[z + 1] - zmw_start[z]) * L;
+  const int64_t off = read_off[z];
+  const int n = (int)(read_off[z + 1] - off);
   const uint8_t* in_b = bases + off;
   const uint8_t* in_q = quals + off;
   uint8_t* out_b = seq_out + off;
@@ -3146,9 +3147,9 @@ stitch_kernel(const uint8_t* __restrict__ bases, const uint8_t* __restrict__ qua
   if (threadIdx.x == 0) len_out[z] = running;
 }
 
-void launch_stitch(const uint8_t* bases, const uint8_t* quals, int L, const int32_t* zmw_start, int n_zmw,
+void launch_stitch(const uint8_t* bases, const uint8_t* quals, const int64_t* read_off, int n_zmw,
                    uint8_t* seq_out, uint8_t* qual_out, int32_t* len_out, cudaStream_t st) {
-  if (n_zmw > 0) stitch_kernel<<<n_zmw, 256, 0, st>>>(bases, quals, L, zmw_start, seq_out, qual_out, len_out);
+  if (n_zmw > 0) stitch_kernel<<<n_zmw, 256, 0, st>>>(bases, quals, read_off, seq_out, qual_out, len_out);
 }
 
 void launch_head(const HeadParams& p, int ntiles, cudaStream_t st) {

@@ -53,20 +53,23 @@ void launch_stack(float* x, int ntiles, int L, int win, const StackParams& p, co
 int read_ffn_trace(unsigned long long* out, int n);
 void launch_head(const HeadParams& p, int ntiles, cudaStream_t st);
 // per-read window concatenation + gap compaction; read z = windows [zmw_start[z], zmw_start[z+1]) (device pointers)
-void launch_stitch(const uint8_t* bases, const uint8_t* quals, int L, const int32_t* zmw_start, int n_zmw,
+// read z spans bytes [read_off[z], read_off[z + 1]) of bases / quals (and of seq_out / qual_out); int64 offsets
+void launch_stitch(const uint8_t* bases, const uint8_t* quals, const int64_t* read_off, int n_zmw,
                    uint8_t* seq_out, uint8_t* qual_out, int32_t* len_out, cudaStream_t st);
 
 
 // ---- post-model stage on the device (post_kernels.cu); outcome codes: DCB_READ_* of include/dcb200.h
-void launch_read_outcome(const uint8_t* qual, const int32_t* len, const int32_t* zmw_start, const int32_t* window_pos,
-                         int L, int n_zmw, const double* p10, double min_quality, int min_length, int32_t* outcome,
+void launch_read_outcome(const uint8_t* qual, const int32_t* len, const int64_t* read_off, const int32_t* zmw_start,
+                         const int32_t* window_pos, int L, int n_zmw, const double* p10, double min_quality, int min_length, int32_t* outcome,
                          double* avg_q, cudaStream_t st);
-void launch_fastq(const uint8_t* seq, const uint8_t* qual, const int32_t* len, const int32_t* zmw_start, int L, int n_zmw,
+void launch_fastq(const uint8_t* seq, const uint8_t* qual, const int32_t* len, const int64_t* read_off, int n_zmw,
                   const int32_t* outcome, const uint8_t* names, const int32_t* name_off, int64_t* rec_off, uint8_t* fastq,
                   int64_t cap, cudaStream_t st);
 void launch_skip_mask(const int16_t* ccs_bq, int n_windows, int L, const double* p10, double thr, uint8_t* mask,
                       double* avg_out, cudaStream_t st);
-void launch_fill_skipped(const uint8_t* ccs_ids, const int16_t* ccs_bq, const int32_t* dst, int k, int L, int calib_enabled,
+// skipped window j: source bytes [src_off[j], src_off[j + 1]) of ccs_ids / ccs_bq -> bytes from dst_off[j] of bases / quals
+void launch_fill_skipped(const uint8_t* ccs_ids, const int16_t* ccs_bq, const int64_t* src_off, const int64_t* dst_off, int k,
+                         int calib_enabled,
                          double thr, double cw, double cb, int max_q, uint8_t* bases, uint8_t* quals, int* status,
                          cudaStream_t st);
 

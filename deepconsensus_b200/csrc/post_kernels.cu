@@ -26,8 +26,8 @@
 namespace dcb {
 
 __global__ void __launch_bounds__(256)
-read_outcome_kernel(const uint8_t* __restrict__ qual, const int32_t* __restrict__ len, const int32_t* __restrict__ zmw_start,
-                    const int32_t* __restrict__ window_pos, int L, const double* __restrict__ p10, double min_quality,
+read_outcome_kernel(const uint8_t* __restrict__ qual, const int32_t* __restrict__ len, const int64_t* __restrict__ read_off,
+                    const int32_t* __restrict__ zmw_start, const int32_t* __restrict__ window_pos, int L, const double* __restrict__ p10, double min_quality,
                     int min_length, int32_t* __restrict__ outcome, double* __restrict__ avg_q_out) {
   __shared__ int s_hist[256];
   __shared__ int s_missing;
@@ -36,17 +36,18 @@ read_outcome_kernel(const uint8_t* __restrict__ qual, const int32_t* __restrict_
   s_hist[threadIdx.x] = 0;
   if (threadIdx.x == 0) s_missing = 0;
   __syncthreads();
-  // get_full_sequence: window i of the read must not start beyond i * max_length (a window is missing otherwise)
+  // get_full_sequence: window i of the read must not start beyond i * max_length (a window is missing otherwise) --
+  // whatever the widths of the windows before it (stitch_utils.py:60-78 advances by max_length per window)
   for (int i = threadIdx.x; i < w1 - w0; i += blockDim.x)
     if (window_pos[w0 + i] > i * L) s_missing = 1;
   const int n = len[z];
-  const uint8_t* q = qual + (size_t)w0 * L;
+  const uint8_t* q = qual + read_off[z];
   for (int i = threadIdx.x; i < n; i += blockDim.x) atomicAdd(&s_hist[q[i]], 1);   // integer atomics: exact
   __syncthreads();
   if (threadIdx.x != 0) return;
   int code;
   double avg_q = 0.0;
-  if (s_missing || w1 == w0 || L == 0) code = DCB_READ_EMPTY;
+  if (s_missing || w1 == w0 || read_off[z + 1] == read_off[z]) code = DCB_READ_EMPTY;   // `not full_seq`
   else if (n == 0) code = DCB_READ_ONLY_GAPS;
   else {
     // quality_string_to_array subtracts 33; entries < 0 are dropped by avg_phred (none can be: chars >= '!')
@@ -97,7 +98,7 @@ fastq_layout_kernel(const int32_t* __restrict__ len, const int32_t* __restrict__
 
 __global__ void __launch_bounds__(256)
 fastq_write_kernel(const uint8_t* __restrict__ seq, const uint8_t* __restrict__ qual, const int32_t* __restrict__ len,
-                   const int32_t* __restrict__ zmw_start, int L, const int32_t* __restrict__ outcome,
+                   const int64_t* __restrict__ read_off, const int32_t* __restrict__ outcome,
                    const uint8_t* __restrict__ names, const int32_t* __restrict__ name_off,
                    const int64_t* __restrict__ rec_off, uint8_t* __restrict__ fastq, int64_t cap) {
   const int z = blockIdx.x;
@@ -105,8 +106,8 @@ fastq_write_kernel(const uint8_t* __restrict__ seq, const uint8_t* __restrict__ 
   const int n = len[z], nl = name_off[z + 1] - name_off[z];
   const int64_t o = rec_off[z];
   if (o + nl + 2ll * n + 6 > cap) return;                  // caller sized the buffer too small: rec_off[n_zmw] tells
-  const uint8_t* s = seq + (size_t)zmw_start[z] * L;
-  const uint8_t* q = qual + (size_t)zmw_start[z] * L;
+  const uint8_t* s = seq + read_off[z];
+  const uint8_t* q = qual + read_off[z];
   const uint8_t* nm = names + name_off[z];
   uint8_t* out = fastq + o;
   if (threadIdx.x == 0) {
@@ -142,15 +143,19 @@ skip_mask_kernel(const int16_t* __restrict__ ccs_bq, int n_windows, int L, const
   if (avg_out) avg_out[w] = avg;
 }
 
-// process_skipped_window for k windows: window j goes to row dst[j] of the [*, L] output arrays
+// process_skipped_window for k windows, one warp per window: window j (source bytes [src_off[j], src_off[j + 1]), max_length
+// of them, or its own width for an overflow window) goes to the output bytes from dst_off[j]
 __global__ void __launch_bounds__(256)
-fill_skipped_kernel(const uint8_t* __restrict__ ccs_ids, const int16_t* __restrict__ ccs_bq, const int32_t* __restrict__ dst,
-                    int k, int L, int calib_enabled, double thr, double cw, double cb, int max_q,
+fill_skipped_kernel(const uint8_t* __restrict__ ccs_ids, const int16_t* __restrict__ ccs_bq,
+                    const int64_t* __restrict__ src_off, const int64_t* __restrict__ dst_off,
+                    int k, int calib_enabled, double thr, double cw, double cb, int max_q,
                     uint8_t* __restrict__ bases, uint8_t* __restrict__ quals, int* __restrict__ status) {
   const char vocab[5] = {' ', 'A', 'T', 'C', 'G'};
-  const long long total = (long long)k * L;
-  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
-    const int j = (int)(i / L), l = (int)(i - (long long)j * L);
+  const int j = blockIdx.x * 8 + (threadIdx.x >> 5);
+  if (j >= k) return;
+  const int64_t s0 = src_off[j], width = src_off[j + 1] - s0, d0 = dst_off[j];
+  for (int64_t l = threadIdx.x & 31; l < width; l += 32) {
+    const int64_t i = s0 + l;
     int id = ccs_ids[i];
     if (id > 4) { atomicOr(status, 1); id = 4; }
     const int qraw = ccs_bq[i];
@@ -165,24 +170,26 @@ fill_skipped_kernel(const uint8_t* __restrict__ ccs_ids, const int16_t* __restri
     } else {
       qi = qraw < max_q ? qraw : max_q;
     }
-    const size_t o = (size_t)dst[j] * L + l;
+    const int64_t o = d0 + l;
     bases[o] = (uint8_t)vocab[id];
     quals[o] = (uint8_t)(qi + 33);                      // quality_scores_to_string (utils.py:60-62)
   }
 }
 
-void launch_read_outcome(const uint8_t* qual, const int32_t* len, const int32_t* zmw_start, const int32_t* window_pos,
-                         int L, int n_zmw, const double* p10, double min_quality, int min_length, int32_t* outcome,
-                         double* avg_q, cudaStream_t st) {
-  if (n_zmw > 0) read_outcome_kernel<<<n_zmw, 256, 0, st>>>(qual, len, zmw_start, window_pos, L, p10, min_quality, min_length, outcome, avg_q);
+void launch_read_outcome(const uint8_t* qual, const int32_t* len, const int64_t* read_off, const int32_t* zmw_start,
+                         const int32_t* window_pos, int L, int n_zmw, const double* p10, double min_quality,
+                         int min_length, int32_t* outcome, double* avg_q, cudaStream_t st) {
+  if (n_zmw > 0)
+    read_outcome_kernel<<<n_zmw, 256, 0, st>>>(qual, len, read_off, zmw_start, window_pos, L, p10, min_quality, min_length,
+                                               outcome, avg_q);
 }
 
-void launch_fastq(const uint8_t* seq, const uint8_t* qual, const int32_t* len, const int32_t* zmw_start, int L, int n_zmw,
+void launch_fastq(const uint8_t* seq, const uint8_t* qual, const int32_t* len, const int64_t* read_off, int n_zmw,
                   const int32_t* outcome, const uint8_t* names, const int32_t* name_off, int64_t* rec_off, uint8_t* fastq,
                   int64_t cap, cudaStream_t st) {
   if (n_zmw <= 0) return;
   fastq_layout_kernel<<<1, 1024, 0, st>>>(len, outcome, name_off, n_zmw, rec_off);
-  fastq_write_kernel<<<n_zmw, 256, 0, st>>>(seq, qual, len, zmw_start, L, outcome, names, name_off, rec_off, fastq, cap);
+  fastq_write_kernel<<<n_zmw, 256, 0, st>>>(seq, qual, len, read_off, outcome, names, name_off, rec_off, fastq, cap);
 }
 
 void launch_skip_mask(const int16_t* ccs_bq, int n_windows, int L, const double* p10, double thr, uint8_t* mask,
@@ -190,13 +197,12 @@ void launch_skip_mask(const int16_t* ccs_bq, int n_windows, int L, const double*
   if (n_windows > 0) skip_mask_kernel<<<(n_windows + 7) / 8, 256, 0, st>>>(ccs_bq, n_windows, L, p10, thr, mask, avg_out);
 }
 
-void launch_fill_skipped(const uint8_t* ccs_ids, const int16_t* ccs_bq, const int32_t* dst, int k, int L, int calib_enabled,
-                         double thr, double cw, double cb, int max_q, uint8_t* bases, uint8_t* quals, int* status,
-                         cudaStream_t st) {
+void launch_fill_skipped(const uint8_t* ccs_ids, const int16_t* ccs_bq, const int64_t* src_off, const int64_t* dst_off, int k,
+                         int calib_enabled, double thr, double cw, double cb, int max_q, uint8_t* bases, uint8_t* quals,
+                         int* status, cudaStream_t st) {
   if (k <= 0) return;
-  const long long total = (long long)k * L;
-  const int grid = (int)((total + 255) / 256 < 1184 ? (total + 255) / 256 : 1184);
-  fill_skipped_kernel<<<grid, 256, 0, st>>>(ccs_ids, ccs_bq, dst, k, L, calib_enabled, thr, cw, cb, max_q, bases, quals, status);
+  fill_skipped_kernel<<<(k + 7) / 8, 256, 0, st>>>(ccs_ids, ccs_bq, src_off, dst_off, k, calib_enabled, thr, cw, cb, max_q,
+                                                    bases, quals, status);
 }
 
 }  // namespace dcb

@@ -78,7 +78,9 @@ ABI_SYMBOLS = (
     "dcb_create", "dcb_load_weights", "dcb_forward", "dcb_submit", "dcb_wait", "dcb_stitch", "dcb_last_forward_ms",
     "dcb_packed_window_bytes", "dcb_pack_rows", "dcb_forward_packed", "dcb_submit_packed",
     "dcb_stitch_fastq", "dcb_skip_mask", "dcb_fill_skipped",
-    "dcb_prep_open", "dcb_prep_set_threads", "dcb_prep_next_zmw", "dcb_prep_get_windows", "dcb_prep_ccs_header", "dcb_prep_close",
+    "dcb_stitch_fastq_ragged", "dcb_fill_skipped_ragged",
+    "dcb_prep_open", "dcb_prep_set_threads", "dcb_prep_set_smart_windows", "dcb_prep_next_zmw", "dcb_prep_get_windows",
+    "dcb_prep_get_window_widths", "dcb_prep_get_overflow_windows", "dcb_prep_ccs_header", "dcb_prep_close",
     "dcb_prep_last_error", "dcb_bamw_open", "dcb_bamw_write", "dcb_bamw_close",
     "dcb_last_forward_launches", "dcb_set_profile", "dcb_get_profile", "dcb_get_profile_kernels", "dcb_alloc_host",
     "dcb_free_host", "dcb_alloc_device", "dcb_free_device", "dcb_memcpy_h2d", "dcb_memcpy_d2h",
@@ -134,6 +136,9 @@ def _load(path: str) -> ctypes.CDLL:
   lib.dcb_stitch_fastq.argtypes = [vp, vp, vp, i32, i32, vp, i32, vp, vp, vp, f64, i32, u32, vp, ctypes.c_int64, vp, vp, vp]
   lib.dcb_skip_mask.argtypes = [vp, vp, i32, i32, f64, vp, vp]
   lib.dcb_fill_skipped.argtypes = [vp, vp, vp, vp, i32, i32, i32, f64, f64, f64, u32, vp, vp]
+  lib.dcb_stitch_fastq_ragged.argtypes = [vp, vp, vp, i32, vp, i32, vp, i32, vp, vp, vp, f64, i32, u32, vp, ctypes.c_int64,
+                                          vp, vp, vp]
+  lib.dcb_fill_skipped_ragged.argtypes = [vp, vp, vp, vp, vp, i32, i32, f64, f64, f64, u32, vp, vp]
   lib.dcb_last_forward_ms.argtypes = [vp, ctypes.POINTER(ctypes.c_float)]
   lib.dcb_last_forward_launches.argtypes = [vp, ctypes.POINTER(i32)]
   lib.dcb_set_debug.argtypes = [vp, i32]
@@ -486,10 +491,13 @@ class B200Model:
     return seq, qual, lens
 
   def stitch_fastq(self, bases, quals, zmw_start: np.ndarray, window_pos, names, min_quality: float, min_length: int,
-                   n_windows: Optional[int] = None, on_device: bool = False, length: Optional[int] = None):
+                   n_windows: Optional[int] = None, on_device: bool = False, length: Optional[int] = None,
+                   window_off: Optional[np.ndarray] = None):
     """dcb_stitch_fastq: stitch_utils.stitch_to_fastq for a batch of reads on the device.  Returns (fastq bytes,
     rec_off int64 [n_zmw + 1], outcome int32 [n_zmw], avg_q float64 [n_zmw]); read z's record is
-    fastq[rec_off[z]:rec_off[z + 1]] (empty unless outcome[z] & 0x7f == DCB_READ_OK)."""
+    fastq[rec_off[z]:rec_off[z + 1]] (empty unless outcome[z] & 0x7f == DCB_READ_OK).
+    window_off (int64 [n_windows + 1], host arrays only): windows of their own width, dcb_stitch_fastq_ragged -- bases /
+    quals are flat and window w is bytes [window_off[w], window_off[w + 1])."""
     zs = np.ascontiguousarray(zmw_start, dtype=np.int32)
     nz = int(zs.shape[0]) - 1
     L = int(length) if length is not None else self.max_length
@@ -502,6 +510,11 @@ class B200Model:
       quals = np.ascontiguousarray(quals, dtype=np.uint8)
       n_windows = int(bases.shape[0])
       b_ptr, q_ptr, flags = bases.ctypes.data_as(ctypes.c_void_p), quals.ctypes.data_as(ctypes.c_void_p), 0
+    if window_off is not None:
+      window_off = np.ascontiguousarray(window_off, dtype=np.int64)
+      n_windows = int(window_off.shape[0]) - 1
+      if on_device or int(window_off[-1]) > min(bases.size, quals.size):
+        raise ValueError("stitch_fastq: window_off needs host arrays that hold window_off[-1] bytes")
     pos = np.ascontiguousarray(window_pos, dtype=np.int32)
     if pos.shape[0] != n_windows:
       raise ValueError("window_pos must have one entry per window")
@@ -512,15 +525,21 @@ class B200Model:
     if nz:
       name_off[1:] = np.cumsum([len(x) for x in enc])
     blob = np.frombuffer(b"".join(enc) or b"\0", np.uint8)
-    cap = int(name_off[-1]) + 2 * n_windows * L + 6 * nz + 16
+    cap = int(name_off[-1]) + 2 * (n_windows * L if window_off is None else int(window_off[-1])) + 6 * nz + 16
     fastq = np.empty(cap, np.uint8)
     rec_off = np.zeros(nz + 1, np.int64)
     outcome = np.zeros(max(nz, 0), np.int32)
     avg_q = np.zeros(max(nz, 0), np.float64)
     vp = lambda a: a.ctypes.data_as(ctypes.c_void_p)
-    self._check(self._lib.dcb_stitch_fastq(self._handle, b_ptr, q_ptr, n_windows, L, vp(zs), nz, vp(pos), vp(blob),
-                                           vp(name_off), float(min_quality), int(min_length), flags, vp(fastq), cap,
-                                           vp(rec_off), vp(outcome), vp(avg_q)))
+    if window_off is None:
+      self._check(self._lib.dcb_stitch_fastq(self._handle, b_ptr, q_ptr, n_windows, L, vp(zs), nz, vp(pos), vp(blob),
+                                             vp(name_off), float(min_quality), int(min_length), flags, vp(fastq), cap,
+                                             vp(rec_off), vp(outcome), vp(avg_q)))
+    else:
+      self._check(self._lib.dcb_stitch_fastq_ragged(self._handle, b_ptr, q_ptr, n_windows, vp(window_off), L, vp(zs), nz,
+                                                    vp(pos), vp(blob), vp(name_off), float(min_quality),
+                                                    int(min_length), flags, vp(fastq), cap, vp(rec_off), vp(outcome),
+                                                    vp(avg_q)))
     return fastq[:int(rec_off[-1])].tobytes(), rec_off, outcome, avg_q
 
   def skip_mask(self, ccs_base_quality_scores: np.ndarray, skip_windows_above: float) -> Tuple[np.ndarray, np.ndarray]:
@@ -560,6 +579,30 @@ class B200Model:
     self._check(self._lib.dcb_fill_skipped(self._handle, vp(ids), vp(bq), vp(dst), k, L, en,
                                            float(cal.threshold) if en else 0.0, float(cal.w) if en else 1.0,
                                            float(cal.b) if en else 0.0, flags, b_ptr, q_ptr))
+
+  def fill_skipped_ragged(self, ccs_ids: np.ndarray, ccs_base_quality_scores: np.ndarray, src_off: np.ndarray,
+                          dst_off: np.ndarray, bases: np.ndarray, quals: np.ndarray,
+                          calibration: Optional[calibration_lib.QualityCalibrationValues] = None) -> None:
+    """dcb_fill_skipped_ragged: `fill_skipped` for windows of their own width.  Window j is entries
+    [src_off[j], src_off[j + 1]) of ccs_ids / ccs_base_quality_scores (flat) and lands at byte dst_off[j] of the flat
+    host uint8 arrays bases / quals."""
+    ids = np.ascontiguousarray(ccs_ids, dtype=np.uint8).reshape(-1)
+    bq = np.ascontiguousarray(ccs_base_quality_scores, dtype=np.int16).reshape(-1)
+    src = np.ascontiguousarray(src_off, dtype=np.int64)
+    dst = np.ascontiguousarray(dst_off, dtype=np.int64)
+    k = int(src.shape[0]) - 1
+    if dst.shape != (k,) or int(src[-1]) > min(ids.shape[0], bq.shape[0]):
+      raise ValueError("fill_skipped_ragged: src_off [k + 1] within ccs_ids / ccs_base_quality_scores and dst_off [k] expected")
+    if not (bases.flags.c_contiguous and quals.flags.c_contiguous and bases.dtype == np.uint8 and quals.dtype == np.uint8):
+      raise ValueError("fill_skipped_ragged: bases / quals must be C-contiguous uint8 arrays")
+    if k and int((dst + np.diff(src)).max()) > min(bases.size, quals.size):
+      raise ValueError("fill_skipped_ragged: destination outside the output arrays")
+    cal = calibration
+    en = int(bool(cal is not None and cal.enabled))
+    vp = lambda a: a.ctypes.data_as(ctypes.c_void_p)
+    self._check(self._lib.dcb_fill_skipped_ragged(self._handle, vp(ids), vp(bq), vp(src), vp(dst), k, en,
+                                                  float(cal.threshold) if en else 0.0, float(cal.w) if en else 1.0,
+                                                  float(cal.b) if en else 0.0, 0, vp(bases), vp(quals)))
 
   def stitch_raw(self, bases_ptr: int, quals_ptr: int, n_windows: int, zmw_start: np.ndarray, flags: int,
                  seq_ptr: int, qual_ptr: int, len_ptr: int, length: Optional[int] = None) -> None:

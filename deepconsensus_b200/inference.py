@@ -183,29 +183,26 @@ def run_model_and_stitch(feature_dicts: List[Dict[str, Any]], model: engine_lib.
     positions.extend(int(x) for x in data["window_pos"])
 
   _pipelined(model, batch_examples(feature_dicts, model_params, options), collect)
-  if skipped_outputs:
-    sb = np.empty((len(skipped_outputs), L), np.uint8)
-    sq = np.empty((len(skipped_outputs), L), np.uint8)
-    for i, o in enumerate(skipped_outputs):
-      seq, qual = o.sequence.encode("latin-1"), o.quality_string.encode("latin-1")
-      if len(seq) != L or len(qual) != L:
-        raise ValueError("skipped window %s@%s is not %d characters long" % (o.molecule_name, o.window_pos, L))
-      sb[i] = np.frombuffer(seq, np.uint8)
-      sq[i] = np.frombuffer(qual, np.uint8)
-      names.append(_as_str(o.molecule_name))
-      positions.append(int(o.window_pos))
-    bases.append(sb)
-    quals.append(sq)
+  widths = [L] * len(names)
+  for o in skipped_outputs or []:                 # an overflow window (CCS smart windows) keeps its own width
+    seq, qual = o.sequence.encode("latin-1"), o.quality_string.encode("latin-1")
+    if len(seq) != len(qual):
+      raise ValueError("skipped window %s@%s: sequence and quality differ in length" % (o.molecule_name, o.window_pos))
+    bases.append(np.frombuffer(seq, np.uint8))
+    quals.append(np.frombuffer(qual, np.uint8))
+    widths.append(len(seq))
+    names.append(_as_str(o.molecule_name))
+    positions.append(int(o.window_pos))
   if not names:
     return []
-  all_b, all_q = np.concatenate(bases), np.concatenate(quals)
   order = sorted(range(len(names)), key=lambda i: (names[i], positions[i]))     # quick_inference.py:721-728
-  if order != list(range(len(names))):
-    all_b, all_q = all_b[order], all_q[order]
-    names = [names[i] for i in order]
-    positions = [positions[i] for i in order]
-  return stitch_gpu.stitch_batch_to_fastq(model, all_b, all_q, names, positions, L, options.min_quality,
-                                          options.min_length, outcome_counter)
+  widths = np.asarray(widths, np.int64)
+  window_off = np.concatenate([[0], np.cumsum(widths[order])])
+  at = _ranges(np.concatenate([[0], np.cumsum(widths)])[order], widths[order])
+  all_b = np.concatenate([b.reshape(-1) for b in bases])[at]
+  all_q = np.concatenate([q.reshape(-1) for q in quals])[at]
+  return stitch_gpu.stitch_batch_to_fastq(model, all_b, all_q, [names[i] for i in order], [positions[i] for i in order], L,
+                                          options.min_quality, options.min_length, outcome_counter, window_off=window_off)
 
 
 def inference_on_zmw_windows(feature_dicts_for_zmws: Iterable[Iterable[Dict[str, Any]]], model: engine_lib.B200Model,
@@ -216,8 +213,8 @@ def inference_on_zmw_windows(feature_dicts_for_zmws: Iterable[Iterable[Dict[str,
 
     skip decision   avg_phred(ccs_base_quality_scores) > skip_windows_above     dcb_skip_mask
     model           run_model_on_examples on the windows that are not skipped    dcb_submit / dcb_wait
-    skipped windows process_skipped_window: adopt CCS bases / calibrated quals    dcb_fill_skipped
-    stitch          sort by (name, window_pos), stitch_to_fastq per read          dcb_stitch_fastq
+    skipped windows process_skipped_window: adopt CCS bases / calibrated quals    dcb_fill_skipped_ragged
+    stitch          sort by (name, window_pos), stitch_to_fastq per read          dcb_stitch_fastq_ragged
 
   Returns one FASTQ record (or None) per read in sorted-name order -- identical to the reference flow built from
   `split_skipped_windows`, `run_model_on_examples`, `sorted(...)` and `stitch_utils.stitch_to_fastq`.
@@ -230,34 +227,37 @@ def inference_on_zmw_windows(feature_dicts_for_zmws: Iterable[Iterable[Dict[str,
     return []
   names = [_as_str(w["name"]) for w in windows]
   positions = [int(w["window_pos"]) for w in windows]
-  bq = np.stack([np.asarray(w["ccs_base_quality_scores"]) for w in windows]).astype(np.int16)
   skip = np.array([bool(w.get("overflow", False)) for w in windows])
-  if options.skip_windows_above:
+  widths = np.array([len(w["ccs_base_quality_scores"]) if o else L for w, o in zip(windows, skip)], np.int64)
+  fit = np.nonzero(~skip)[0]                                  # overflow windows are skipped before the quality decision
+  if options.skip_windows_above and len(fit):
+    bq = np.stack([np.asarray(windows[i]["ccs_base_quality_scores"]) for i in fit]).astype(np.int16)
     mask, _ = model.skip_mask(bq, options.skip_windows_above)
     for i in np.nonzero(mask == 2)[0]:                       # within 1e-7 of the threshold: the reference's expression
-      mask[i] = utils.avg_phred(windows[i]["ccs_base_quality_scores"]) > options.skip_windows_above
-    skip |= mask.astype(bool)
+      mask[i] = utils.avg_phred(windows[fit[i]]["ccs_base_quality_scores"]) > options.skip_windows_above
+    skip[fit] |= mask.astype(bool)
   order = sorted(range(n), key=lambda i: (names[i], positions[i]))          # quick_inference.py:721-728
-  dest = np.empty(n, np.int32)
-  dest[order] = np.arange(n, dtype=np.int32)
-  all_b, all_q = np.empty((n, L), np.uint8), np.empty((n, L), np.uint8)
+  dest = np.empty(n, np.int64)
+  dest[order] = np.arange(n)
+  window_off, all_b, all_q = _window_layout(widths, dest)
   scored = np.nonzero(~skip)[0]
   cursor = [0]
 
   def collect(data, out):
     k = out["bases"].shape[0]
-    rows = dest[scored[cursor[0]:cursor[0] + k]]
-    all_b[rows], all_q[rows] = out["bases"], out["quals"]
+    _place(all_b, all_q, window_off, dest[scored[cursor[0]:cursor[0] + k]], out, L)
     cursor[0] += k
 
   _pipelined(model, batch_examples([windows[i] for i in scored], model_params, options), collect)
   skipped = np.nonzero(skip)[0]
   if len(skipped):
     ccs_row = params_lib.get_indices(options.max_passes, options.use_ccs_bq)[4][0]
-    ccs_ids = np.stack([np.asarray(windows[i]["subreads"])[ccs_row, :, 0] for i in skipped]).astype(np.uint8)
-    model.fill_skipped(ccs_ids, bq[skipped], dest[skipped], all_b, all_q, calibration=options.ccs_calibration_values)
+    ccs_ids = np.concatenate([np.asarray(windows[i]["subreads"])[ccs_row, :, 0] for i in skipped]).astype(np.uint8)
+    bq = np.concatenate([np.asarray(windows[i]["ccs_base_quality_scores"]) for i in skipped]).astype(np.int16)
+    model.fill_skipped_ragged(ccs_ids, bq, np.concatenate([[0], np.cumsum(widths[skipped])]), window_off[dest[skipped]],
+                              all_b, all_q, calibration=options.ccs_calibration_values)
   return stitch_gpu.stitch_batch_to_fastq(model, all_b, all_q, [names[i] for i in order], [positions[i] for i in order],
-                                          L, options.min_quality, options.min_length, outcome_counter)
+                                          L, options.min_quality, options.min_length, outcome_counter, window_off=window_off)
 
 
 def inference_on_packed_zmws(zmws: List[Dict[str, Any]], model: engine_lib.B200Model, model_params: params_lib.Params,
@@ -278,36 +278,70 @@ def inference_on_packed_zmws(zmws: List[Dict[str, Any]], model: engine_lib.B200M
   packed = np.concatenate([z["packed"] for z in zmws])
   pos = np.concatenate([z["window_pos"] for z in zmws]).astype(np.int64)
   bq = np.concatenate([z["ccs_bq"] for z in zmws])
-  skip = np.concatenate([z["overflow"] for z in zmws]).astype(bool)
+  over = np.concatenate([z["overflow"] for z in zmws]).astype(bool)
+  widths = np.where(over, np.concatenate([z["widths"] for z in zmws]), L).astype(np.int64)
+  skip = over.copy()
   counts = np.array([len(z["window_pos"]) for z in zmws])
   names_z = [z["name"] for z in zmws]
   n = len(pos)
-  if options.skip_windows_above:
-    mask, _ = model.skip_mask(bq, options.skip_windows_above)
+  fit = np.nonzero(~over)[0]                                  # overflow windows are skipped before the quality decision
+  if options.skip_windows_above and len(fit):
+    mask, _ = model.skip_mask(bq[fit], options.skip_windows_above)
     for i in np.nonzero(mask == 2)[0]:
-      mask[i] = utils.avg_phred(bq[i].astype(np.int64)) > options.skip_windows_above
-    skip |= mask.astype(bool)
+      mask[i] = utils.avg_phred(bq[fit[i]].astype(np.int64)) > options.skip_windows_above
+    skip[fit] |= mask.astype(bool)
   # sort by (name, window_pos): ZMW order by name, windows inside a ZMW by position (quick_inference.py:721-728)
   zorder = sorted(range(len(zmws)), key=lambda k: names_z[k])
   starts = np.concatenate([[0], np.cumsum(counts)])
   order = np.concatenate([starts[k] + np.argsort(pos[starts[k]:starts[k + 1]], kind="stable") for k in zorder])
   dest = np.empty(n, np.int64)
   dest[order] = np.arange(n)
-  all_b, all_q = np.empty((n, L), np.uint8), np.empty((n, L), np.uint8)
+  window_off, all_b, all_q = _window_layout(widths, dest)
   scored = np.nonzero(~skip)[0]
   for b0 in range(0, len(scored), options.batch_size):          # batch_examples (quick_inference.py:304-338)
     idx = scored[b0:b0 + options.batch_size]
-    out = model.forward_packed(packed[idx])
-    all_b[dest[idx]], all_q[dest[idx]] = out["bases"], out["quals"]
+    _place(all_b, all_q, window_off, dest[idx], model.forward_packed(packed[idx]), L)
   skipped = np.nonzero(skip)[0]
   if len(skipped):
-    ccs_ids = packed[skipped][:, 3 * P * L:3 * P * L + L]        # the CCS plane of the packed rows
-    model.fill_skipped(ccs_ids, bq[skipped], dest[skipped].astype(np.int32), all_b, all_q,
-                       calibration=options.ccs_calibration_values)
+    # CCS ids / qualities of the skipped windows back to back: the CCS plane of the packed rows and ccs_bq for windows
+    # that fit, the wide arrays of next_zmw for overflow windows (which come in window order)
+    start = np.arange(n, dtype=np.int64) * L
+    start[over] = n * L + np.concatenate([[0], np.cumsum(widths[over])])[:-1]
+    at = _ranges(start[skipped], widths[skipped])
+    ccs_ids = np.concatenate([packed[:, 3 * P * L:3 * P * L + L].reshape(-1)] + [z["wide_ccs_ids"] for z in zmws])[at]
+    ccs_bq = np.concatenate([bq.reshape(-1)] + [z["wide_ccs_bq"] for z in zmws])[at]
+    model.fill_skipped_ragged(ccs_ids, ccs_bq, np.concatenate([[0], np.cumsum(widths[skipped])]),
+                              window_off[dest[skipped]], all_b, all_q, calibration=options.ccs_calibration_values)
   names_sorted = [names_z[k] for k in zorder for _ in range(counts[k])]
   fastq, rec_off, passed = stitch_gpu.stitch_batch_to_fastq_bytes(model, all_b, all_q, names_sorted, pos[order].tolist(), L,
-                                                                  options.min_quality, options.min_length, outcome_counter)
+                                                                  options.min_quality, options.min_length, outcome_counter,
+                                                                  window_off=window_off)
   return fastq, rec_off, passed, [names_z[k] for k in zorder]
+
+
+# Windows of their own width (CCS smart windows: an overflow window keeps all W columns): the post-model stage holds
+# every window's bytes back to back in sorted order and addresses them through int64 offsets.
+def _window_layout(widths: np.ndarray, dest: np.ndarray) -> Tuple[np.ndarray, np.ndarray, np.ndarray]:
+  """(window_off [n + 1], bases, quals) for windows whose sorted position is dest[i]."""
+  sorted_widths = np.empty(len(widths), np.int64)
+  sorted_widths[dest] = widths
+  window_off = np.concatenate([[0], np.cumsum(sorted_widths)])
+  return window_off, np.empty(int(window_off[-1]), np.uint8), np.empty(int(window_off[-1]), np.uint8)
+
+
+def _place(all_b: np.ndarray, all_q: np.ndarray, window_off: np.ndarray, rows: np.ndarray, out: Dict[str, Any], L: int):
+  """The model's [k, L] outputs into sorted windows `rows`."""
+  if window_off[-1] == L * (len(window_off) - 1):             # every window L wide: whole rows
+    all_b.reshape(-1, L)[rows], all_q.reshape(-1, L)[rows] = out["bases"], out["quals"]
+  else:
+    at = window_off[rows][:, None] + np.arange(L)
+    all_b[at], all_q[at] = out["bases"], out["quals"]
+
+
+def _ranges(start: np.ndarray, widths: np.ndarray) -> np.ndarray:
+  """Indices start[j] .. start[j] + widths[j] - 1 for every j, back to back."""
+  off = np.concatenate([[0], np.cumsum(widths)])
+  return np.repeat(np.asarray(start, np.int64) - off[:-1], widths) + np.arange(off[-1])
 
 
 def _as_str(x) -> str:

@@ -41,6 +41,9 @@ def _lib():
     vp, i32 = ctypes.c_void_p, ctypes.c_int32
     lib.dcb_prep_open.argtypes = [ctypes.c_char_p, ctypes.c_char_p, i32, i32, i32, i32, ctypes.POINTER(vp)]
     lib.dcb_prep_set_threads.argtypes = [vp, i32]
+    lib.dcb_prep_set_smart_windows.argtypes = [vp, i32]
+    lib.dcb_prep_get_window_widths.argtypes = [vp, vp]
+    lib.dcb_prep_get_overflow_windows.argtypes = [vp, vp, vp, vp]
     lib.dcb_prep_next_zmw.argtypes = [vp, ctypes.POINTER(DcbZmwInfo)]
     lib.dcb_prep_get_windows.argtypes = [vp, vp, vp, vp, vp, vp, vp]
     lib.dcb_prep_ccs_header.argtypes = [vp]
@@ -60,9 +63,11 @@ class BamFeatureStream:
   iter_examples, pre_lib.py:1279-1384,625-697)."""
 
   def __init__(self, subreads_to_ccs: str, ccs_bam: str, max_passes: int, max_length: int, use_ccs_bq: bool = False,
-               ins_trim: int = 5, threads: int = 0):
+               ins_trim: int = 5, threads: int = 0, use_ccs_smart_windows: bool = False):
     """threads > 0: ZMWs are processed by that many native worker threads (plus one BAM-decoding thread) while the
-    caller consumes them; the order of the ZMWs is the file's either way (`--cpus` of `deepconsensus run`)."""
+    caller consumes them; the order of the ZMWs is the file's either way (`--cpus` of `deepconsensus run`).
+    use_ccs_smart_windows: window widths come from the CCS records' `wl` tags (`--use_ccs_smart_windows`); windows
+    wider than max_length are overflow windows, handed out in full by `next_zmw`."""
     self._lib = _lib()
     self._h = ctypes.c_void_p()
     self.max_passes, self.max_length, self.use_ccs_bq = int(max_passes), int(max_length), bool(use_ccs_bq)
@@ -72,6 +77,8 @@ class BamFeatureStream:
     if rc:
       raise PrepError(self._lib.dcb_prep_last_error().decode("utf-8", "replace"))
     if threads > 0 and self._lib.dcb_prep_set_threads(self._h, int(threads)):
+      raise PrepError(self._lib.dcb_prep_last_error().decode("utf-8", "replace"))
+    if use_ccs_smart_windows and self._lib.dcb_prep_set_smart_windows(self._h, 1):
       raise PrepError(self._lib.dcb_prep_last_error().decode("utf-8", "replace"))
     self._stride = ((3 * self.max_passes + 1 + int(self.use_ccs_bq)) * self.max_length + 15) // 16 * 16 + 16   # PackedLayout
 
@@ -96,7 +103,10 @@ class BamFeatureStream:
 
   def next_zmw(self, want_rows: bool = True, want_packed: bool = False) -> Optional[Dict[str, Any]]:
     """The next ZMW's windows as arrays: dict(name, n_subreads, ec, np_num_passes, rq, rg, window_pos [n], overflow
-    [n], num_passes [n], ccs_bq int16 [n, L], rows float32 [n, R, L] and / or packed uint8 [n, stride]); None at EOF."""
+    [n], num_passes [n], widths [n] (spaced width W of every window), ccs_bq int16 [n, L], rows float32 [n, R, L] and / or
+    packed uint8 [n, stride]); None at EOF.  Overflow windows (W > L, smart windows only) hold their first L columns in
+    those arrays and come in full, ragged in window order, as wide_ccs_ids uint8 [S], wide_ccs_bq int16 [S] and, with
+    want_rows, wide_rows float32 [S * R] (window after window, each [R, W]; S = sum of their widths)."""
     info = DcbZmwInfo()
     rc = self._lib.dcb_prep_next_zmw(self._h, ctypes.byref(info))
     if rc < 0:
@@ -121,6 +131,17 @@ class BamFeatureStream:
                                         vp(out["overflow"]), vp(out["ccs_bq"]), vp(out["num_passes"]))
     if rc:
       raise PrepError(self._lib.dcb_prep_last_error().decode("utf-8", "replace"))
+    out["widths"] = np.zeros(n, np.int32)
+    self._lib.dcb_prep_get_window_widths(self._h, vp(out["widths"]))
+    wide = int(out["widths"][out["overflow"] != 0].sum())
+    out["wide_ccs_ids"], out["wide_ccs_bq"] = np.zeros(wide, np.uint8), np.zeros(wide, np.int16)
+    if want_rows:
+      out["wide_rows"] = np.zeros(wide * R, np.float32)
+    if wide:
+      rc = self._lib.dcb_prep_get_overflow_windows(self._h, vp(out["wide_rows"]) if want_rows else None,
+                                                   vp(out["wide_ccs_ids"]), vp(out["wide_ccs_bq"]))
+      if rc:
+        raise PrepError(self._lib.dcb_prep_last_error().decode("utf-8", "replace"))
     return out
 
   def __iter__(self):
@@ -132,15 +153,25 @@ class BamFeatureStream:
 
 
 def stream_zmw_windows(subreads_to_ccs: str, ccs_bam: str, max_passes: int, max_length: int, use_ccs_bq: bool = False,
-                       ins_trim: int = 5, limit: int = 0) -> Iterator[List[Dict[str, Any]]]:
-  """Per ZMW, the feature dicts `quick_inference.preprocess` returns (keys of DcExample.to_features_dict)."""
-  stream = BamFeatureStream(subreads_to_ccs, ccs_bam, max_passes, max_length, use_ccs_bq, ins_trim)
+                       ins_trim: int = 5, limit: int = 0, use_ccs_smart_windows: bool = False
+                       ) -> Iterator[List[Dict[str, Any]]]:
+  """Per ZMW, the feature dicts `quick_inference.preprocess` returns (keys of DcExample.to_features_dict).  An overflow
+  window (smart windows only) has subreads [R, W, 1] and W CCS base qualities, as the reference leaves it unpadded."""
+  stream = BamFeatureStream(subreads_to_ccs, ccs_bam, max_passes, max_length, use_ccs_bq, ins_trim,
+                            use_ccs_smart_windows=use_ccs_smart_windows)
   try:
     done = 0
     for z in stream:
-      yield [dict(subreads=z["rows"][i][..., None], **{"subreads/num_passes": int(z["num_passes"][i])},
+      rows, bq = list(z["rows"]), list(z["ccs_bq"])
+      off = 0
+      for i in np.nonzero(z["overflow"])[0]:
+        w = int(z["widths"][i])
+        rows[i] = z["wide_rows"][off * stream.total_rows:(off + w) * stream.total_rows].reshape(stream.total_rows, w)
+        bq[i] = z["wide_ccs_bq"][off:off + w]
+        off += w
+      yield [dict(subreads=rows[i][..., None], **{"subreads/num_passes": int(z["num_passes"][i])},
                   name=z["name"], window_pos=int(z["window_pos"][i]),
-                  ccs_base_quality_scores=z["ccs_bq"][i].astype(np.int64), overflow=bool(z["overflow"][i]),
+                  ccs_base_quality_scores=bq[i].astype(np.int64), overflow=bool(z["overflow"][i]),
                   ec=z["ec"], np_num_passes=z["np_num_passes"], rq=z["rq"], rg=z["rg"])
              for i in range(len(z["window_pos"]))]
       done += 1

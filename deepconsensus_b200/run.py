@@ -2,7 +2,8 @@
 BAM + CCS BAM in, polished reads (FASTQ or unaligned BAM) out.
 
   python -m deepconsensus_b200.run --subreads_to_ccs S.bam --ccs_bam C.bam --checkpoint model_dir/checkpoint-50 \\
-         --output out.fastq [--batch_zmws 100 --batch_size 1024 --min_quality 20 --skip_windows_above 45 ...]
+         --output out.fastq [--batch_zmws 100 --batch_size 1024 --min_quality 20 --skip_windows_above 45
+         --use_ccs_smart_windows ...]
 
 Stages (all but the driver loop in native code): feature construction from BAM (csrc/bam_prep.cpp), skip decision,
 model, skipped-window fill, sort, stitch + filters + FASTQ bytes (CUDA, `inference.inference_on_zmw_windows`), output
@@ -30,9 +31,12 @@ from deepconsensus_b200 import weights as weights_lib
 def run(subreads_to_ccs: str, ccs_bam: str, checkpoint: str, output: str, batch_zmws: int = 100, batch_size: int = 1024,
         min_quality: int = 20, min_length: int = 0, skip_windows_above: int = 45, ins_trim: int = 5,
         max_base_quality: int = 93, dc_calibration: Optional[str] = None, ccs_calibration: str = "skip",
-        limit: int = 0, random_weights: Optional[int] = None, precision: str = "bf16", device: int = 0, cpus: int = 0
-        ) -> stitch_utils.OutcomeCounter:
-  """One inference run; returns the OutcomeCounter (quick_inference.run's return value)."""
+        limit: int = 0, random_weights: Optional[int] = None, precision: str = "bf16", device: int = 0, cpus: int = 0,
+        use_ccs_smart_windows: bool = False) -> stitch_utils.OutcomeCounter:
+  """One inference run; returns the OutcomeCounter (quick_inference.run's return value).
+
+  use_ccs_smart_windows: window widths come from the `wl` tag of every CCS record (quick_inference.py:113-120); windows
+  wider than max_length bypass the model with the CCS call."""
   params = params_lib.read_params_from_json(checkpoint)
   if dc_calibration is None:
     dc_calibration = params.get("dc_calibration", "skip")                      # quick_inference.py:817-831
@@ -49,7 +53,8 @@ def run(subreads_to_ccs: str, ccs_bam: str, checkpoint: str, output: str, batch_
   model, params = inference.initialize_model(checkpoint, params, options, weights=weights, device=device, precision=precision)
   counter = stitch_utils.OutcomeCounter()
   stream = preprocess.BamFeatureStream(subreads_to_ccs, ccs_bam, options.max_passes, options.max_length,
-                                       options.use_ccs_bq, ins_trim, threads=cpus)
+                                       options.use_ccs_bq, ins_trim, threads=cpus,
+                                       use_ccs_smart_windows=use_ccs_smart_windows)
   as_bam = output.endswith(".bam")
   writer: Any = preprocess.BamWriter(output, stream.ccs_header) if as_bam else open(output, "wb")
   stats = dict(zmws=0, windows=0, seconds_features=0.0, seconds_model_and_stitch=0.0)
@@ -113,6 +118,8 @@ def main(argv: Optional[List[str]] = None) -> None:
   ap.add_argument("--random_weights", type=int, default=None)
   ap.add_argument("--precision", default="bf16", choices=["bf16", "fp32"])
   ap.add_argument("--cpus", type=int, default=0, help="native feature-construction threads (0: on the calling thread)")
+  ap.add_argument("--use_ccs_smart_windows", action="store_true",
+                  help="window widths from the CCS records' wl tag instead of max_length columns")
   a = ap.parse_args(argv)
   c = run(**vars(a))
   print(json.dumps(c.__dict__))

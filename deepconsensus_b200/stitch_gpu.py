@@ -35,14 +35,18 @@ def group_reads(molecule_names: Sequence[str]) -> np.ndarray:
 def stitch_batch_to_fastq_bytes(model, bases, quals, molecule_names: Sequence[str], window_pos: Sequence[int],
                                 max_length: int, min_quality: int, min_length: int,
                                 outcome_counter: stitch_utils.OutcomeCounter,
-                                n_windows: Optional[int] = None, on_device: bool = False
-                                ) -> Tuple[bytes, np.ndarray, np.ndarray]:
-  """(fastq bytes, rec_off, passed): read z's record is fastq[rec_off[z]:rec_off[z + 1]] when passed[z]."""
+                                n_windows: Optional[int] = None, on_device: bool = False,
+                                window_off: Optional[np.ndarray] = None) -> Tuple[bytes, np.ndarray, np.ndarray]:
+  """(fastq bytes, rec_off, passed): read z's record is fastq[rec_off[z]:rec_off[z + 1]] when passed[z].
+
+  window_off (int64 [n_windows + 1]): the ragged form for windows of their own width (CCS smart windows): `bases` /
+  `quals` are flat host arrays and window w is bytes [window_off[w], window_off[w + 1]) (dcb_stitch_fastq_ragged)."""
   zs = group_reads(molecule_names)
   nz = len(zs) - 1
   names = [molecule_names[int(zs[z])] for z in range(nz)]
   fastq, rec_off, outcome, _ = model.stitch_fastq(bases, quals, zs, window_pos, names, min_quality, min_length,
-                                                  n_windows=n_windows, on_device=on_device, length=max_length)
+                                                  n_windows=n_windows, on_device=on_device, length=max_length,
+                                                  window_off=window_off)
   passed = np.zeros(nz, bool)
   for z in range(nz):
     code = int(outcome[z])
@@ -52,6 +56,10 @@ def stitch_batch_to_fastq_bytes(model, bases, quals, molecule_names: Sequence[st
       rec = fastq[int(rec_off[z]):int(rec_off[z + 1])] if code == engine_lib.DCB_READ_OK else None
       if rec is not None:
         qual = rec.split(b"\n")[3]
+      elif window_off is not None:            # too short, ragged host arrays: remove_gaps in NumPy
+        a, b = int(window_off[zs[z]]), int(window_off[zs[z + 1]])
+        seg_b, seg_q = np.asarray(bases).reshape(-1)[a:b], np.asarray(quals).reshape(-1)[a:b]
+        qual = seg_q[seg_b != ord(" ")].tobytes()
       else:                                   # too short: the record was not written; recompute from the windows
         qual = _read_quality_bytes(model, bases, quals, zs, z, max_length, n_windows, on_device)
       ok = round(utils.avg_phred(np.frombuffer(qual, np.uint8).astype(np.int64) - 33), 5) >= min_quality
@@ -80,13 +88,16 @@ def _read_quality_bytes(model, bases, quals, zs, z, max_length, n_windows, on_de
 def stitch_batch_to_fastq(model, bases, quals, molecule_names: Sequence[str], window_pos: Sequence[int],
                           max_length: int, min_quality: int, min_length: int,
                           outcome_counter: stitch_utils.OutcomeCounter,
-                          n_windows: Optional[int] = None, on_device: bool = False) -> List[Optional[str]]:
+                          n_windows: Optional[int] = None, on_device: bool = False,
+                          window_off: Optional[np.ndarray] = None) -> List[Optional[str]]:
   """One FASTQ record (or None) per read, for windows grouped by read and sorted by window position.
 
   `bases` / `quals`: uint8 [n_windows, max_length] arrays as `B200Model.forward` returns them, or device addresses
-  of the same (`on_device=True`, e.g. the DCB_OUT_ON_DEVICE outputs of `forward_raw`).
+  of the same (`on_device=True`, e.g. the DCB_OUT_ON_DEVICE outputs of `forward_raw`); with `window_off`, flat host
+  arrays of windows of their own width (see stitch_batch_to_fastq_bytes).
   """
   fastq, rec_off, passed = stitch_batch_to_fastq_bytes(model, bases, quals, molecule_names, window_pos, max_length,
-                                                       min_quality, min_length, outcome_counter, n_windows, on_device)
+                                                       min_quality, min_length, outcome_counter, n_windows, on_device,
+                                                       window_off)
   return [fastq[int(rec_off[z]):int(rec_off[z + 1])].decode("latin-1") if passed[z] else None
           for z in range(len(passed))]

@@ -193,6 +193,18 @@ int dcb_stitch_fastq(dcb_engine* e, const uint8_t* bases, const uint8_t* quals, 
                      uint32_t flags, uint8_t* fastq_out, int64_t fastq_cap, int64_t* rec_off, int32_t* outcome,
                      double* avg_q);
 
+/* dcb_stitch_fastq for windows of their own width (CCS smart windows, dcb_prep_set_smart_windows): window w is the bytes
+ * [window_off[w], window_off[w + 1]) of bases / quals -- max_length bytes for a scored window, W bytes for an overflow
+ * window -- laid out back to back in sorted order; window_off int64 [n_windows + 1], non-decreasing.  L (max_length)
+ * still drives the missing-window check: window i of a read must not start beyond i * L, whatever the widths of the
+ * windows before it (stitch_utils.py:60-78).  fastq_out: names + 2 * window_off[n_windows] + 6 * n_zmw bytes suffice.
+ * Everything else as dcb_stitch_fastq. */
+int dcb_stitch_fastq_ragged(dcb_engine* e, const uint8_t* bases, const uint8_t* quals, int32_t n_windows,
+                            const int64_t* window_off, int32_t L, const int32_t* zmw_start, int32_t n_zmw,
+                            const int32_t* window_pos, const uint8_t* names, const int32_t* name_off, double min_quality,
+                            int32_t min_length, uint32_t flags, uint8_t* fastq_out, int64_t fastq_cap, int64_t* rec_off,
+                            int32_t* outcome, double* avg_q);
+
 /* The skip decision of inference_on_n_zmws (quick_inference.py:663-672) for a batch of windows:
  * mask[w] = avg_phred(ccs_bq[w, :]) > skip_windows_above (entries < 0 are spacing and are dropped, utils.py:88-106);
  * 2 = within 1e-7 of the threshold, caller decides.  ccs_bq: host int16 [n_windows, L]. */
@@ -207,6 +219,12 @@ int dcb_skip_mask(dcb_engine* e, const int16_t* ccs_bq, int32_t n_windows, int32
 int dcb_fill_skipped(dcb_engine* e, const uint8_t* ccs_ids, const int16_t* ccs_bq, const int32_t* dst_window, int32_t k,
                      int32_t L, int32_t calibration_enabled, double calibration_threshold, double calibration_w,
                      double calibration_b, uint32_t flags, uint8_t* bases, uint8_t* quals);
+/* dcb_fill_skipped for windows of their own width (an overflow window keeps all W columns, quick_inference.py:567-594):
+ * window j is the entries [src_off[j], src_off[j + 1]) of ccs_ids (u8) / ccs_bq (int16), src_off int64 [k + 1] with
+ * src_off[0] = 0, and lands at byte dst_off[j] (int64 [k]) of bases / quals. */
+int dcb_fill_skipped_ragged(dcb_engine* e, const uint8_t* ccs_ids, const int16_t* ccs_bq, const int64_t* src_off,
+                            const int64_t* dst_off, int32_t k, int32_t calibration_enabled, double calibration_threshold,
+                            double calibration_w, double calibration_b, uint32_t flags, uint8_t* bases, uint8_t* quals);
 
 /* ---- feature construction from BAM (SURVEY.md section 8(f)3; host C++, htslib-free, needs no GPU) -----------------------
  * What `deepconsensus run` does in front of the model: stream the subreads-to-CCS BAM ZMW by ZMW (SubreadGrouper,
@@ -230,11 +248,25 @@ int dcb_prep_open(const char* subreads_to_ccs_bam, const char* ccs_bam, int32_t 
 /* Process ZMWs on n_threads worker threads plus one BAM-decoding thread (results still come out in file order); call
  * before the first dcb_prep_next_zmw.  n_threads <= 0: everything on the calling thread. */
 int dcb_prep_set_threads(dcb_prep* p, int32_t n_threads);
+/* CCS smart windows (`deepconsensus run --use_ccs_smart_windows`, pre_lib.py:625-650,1329-1331): enable != 0 cuts every
+ * ZMW into windows whose widths, in CCS bases, come from the CCS record's `wl` tag (a B array of any integer subtype)
+ * instead of into max_length columns.  A window's spaced width W (its columns once space_out_subreads has opened gap
+ * columns) may exceed max_length: such an overflow window bypasses the model and keeps all W columns.  A CCS record
+ * without an integer `wl` array, or whose `wl` does not partition the CCS read exactly, is an error (DCB_ERR_INVALID,
+ * message names the read).  Call before the first dcb_prep_next_zmw; off by default. */
+int dcb_prep_set_smart_windows(dcb_prep* p, int32_t enable);
 int dcb_prep_next_zmw(dcb_prep* p, dcb_zmw_info* info);   /* 1 = a ZMW is loaded, 0 = end of file, < 0 = error */
 /* The windows of the loaded ZMW; every output may be NULL.  rows float32 [n, R, L]; packed [n, dcb_packed_window_bytes];
- * window_pos / num_passes int32 [n]; overflow u8 [n]; ccs_bq int16 [n, L] (-1 at gaps and padding). */
+ * window_pos / num_passes int32 [n]; overflow u8 [n] (1 = spaced width > max_length, smart windows only); ccs_bq int16
+ * [n, L] (-1 at gaps and padding).  An overflow window holds its first L columns here (never scored). */
 int dcb_prep_get_windows(dcb_prep* p, float* rows, uint8_t* packed, int32_t* window_pos, uint8_t* overflow,
                          int16_t* ccs_bq, int32_t* num_passes);
+/* widths int32 [n]: the spaced width W of every window of the loaded ZMW (max_length for fixed-width windows). */
+int dcb_prep_get_window_widths(dcb_prep* p, int32_t* widths);
+/* The overflow windows of the loaded ZMW in full, in window order, ragged (each window's W columns back to back, S = the
+ * sum of their widths); every output may be NULL.  rows float32 [R, W] per window (S * R floats in all); ccs_ids u8 [S]
+ * (CCS base ids 0..4); ccs_bq int16 [S] (-1 at gaps). */
+int dcb_prep_get_overflow_windows(dcb_prep* p, float* rows, uint8_t* ccs_ids, int16_t* ccs_bq);
 const char* dcb_prep_ccs_header(dcb_prep* p);             /* SAM header text of the CCS BAM */
 void dcb_prep_close(dcb_prep* p);
 const char* dcb_prep_last_error(void);
