@@ -29,11 +29,9 @@ thread_local std::string g_create_error;
 
 struct LayerDev {
   __nv_bfloat16* wqkv = nullptr;  // 2 groups x [36][432][8]
-  uint8_t* wqkv2 = nullptr;       // 9 groups x [36][96][8] (qkv2_kernel)
   uint8_t* wq3 = nullptr;         // stack kernel: per (head, rank, q|k|v) [36][72][8]
   uint8_t* wqa = nullptr;         // fused QKV+attention: per (head, rank) [36][216][8], rows = q|k|v halves
   __nv_bfloat16* wo = nullptr;    // [36][288][8]
-  uint8_t* wffn = nullptr;        // per ff chunk: [36][128][8] then [16][288][8]
   uint8_t* wffn2 = nullptr;       // CTA-pair image: per (chunk, rank): [36][64][8] then [16][144][8]
   float b2_mean = 0.f;            // mean of b2 over its 280 columns (stack kernel, deferred LayerNorm)
   uint8_t* wffn2s = nullptr;      // the stack kernel's copy: b1 / deferred-LayerNorm terms in the padding rows (common.h, StackParams)
@@ -76,7 +74,6 @@ struct dcb_engine {
   int64_t next_ticket = 0;
   bool weights_loaded = false;
   bool debug = false;
-  bool ffn_pair = true;
   bool fuse_oproj = true;
   bool fuse_embed = true;
   bool fuse_qa = true;
@@ -84,7 +81,6 @@ struct dcb_engine {
                            // gamma * Wfc table in the idle staging area): +1.7 % against the separate head_kernel, and the
                            // residual image is never written back.  DCB_FUSE_HEAD=0 (developer build): head_kernel
   bool stack = true;   // whole encoder stack in one launch (stack_pair_kernel) when the configuration allows it
-  bool qkv2 = false;   // measured: not faster than gemm_kernel<3,QKV> (both sit on the per-SM L2 port), kept as an option
   bool fused_last = false;
   bool stack_last = false;
   bool profile = false;
@@ -258,9 +254,7 @@ int dcb_create(const dcb_config* cfg, dcb_engine** out) {
   // Developer build only (libdcb200_dev.so, csrc/build.sh): environment switches that select the measured
   // alternative kernel paths.  The product library ignores the environment.
   if (const char* env = getenv("DCB_ALIGN")) align = atoi(env) != 0;
-  if (const char* env = getenv("DCB_FFN_PAIR")) e->ffn_pair = atoi(env) != 0;
   if (const char* env = getenv("DCB_FUSE_OPROJ")) e->fuse_oproj = atoi(env) != 0;
-  if (const char* env = getenv("DCB_QKV2")) e->qkv2 = atoi(env) != 0;
   if (const char* env = getenv("DCB_FUSE_EMBED")) e->fuse_embed = atoi(env) != 0;
   if (const char* env = getenv("DCB_FUSE_QA")) e->fuse_qa = atoi(env) != 0;
   if (const char* env = getenv("DCB_STACK")) e->stack = atoi(env) != 0;
@@ -531,23 +525,6 @@ int dcb_load_weights(dcb_engine* e, const dcb_tensor* tensors, int32_t n) {
         img.insert(img.end(), part.begin(), part.end());
       }
       if ((rc = upload(e, &ld.wqkv, img))) return rc;
-      // 9 column groups of 96 for qkv2_kernel
-      std::vector<__nv_bfloat16> img9;
-      for (int grp = 0; grp < kQKVN / 96; ++grp) {
-        auto part = pack_b(kDP, 96, [&](int k, int nn) {
-          const int colg = grp * 96 + nn;
-          const int slot = colg / kDHP, dd = colg % kDHP;
-          if (k >= kD || dd >= kDH) return 0.f;
-          const int proj = slot / kHeads, head = slot % kHeads;
-          const float* w = proj == 0 ? wq : (proj == 1 ? wk : wv);
-          const float v = w[((size_t)k * kHeads + head) * kDH + dd];
-          return proj == 0 ? v * qscale : v;
-        });
-        img9.insert(img9.end(), part.begin(), part.end());
-      }
-      __nv_bfloat16* dptr = nullptr;
-      if ((rc = upload(e, &dptr, img9))) return rc;
-      ld.wqkv2 = reinterpret_cast<uint8_t*>(dptr);
       // fused QKV + attention (CTA pairs): for head h and rank rk the 216 rows of a k-step are
       // [q_h | k_h | v_h], each the rk-th half (72 columns) of that 144-wide matrix
       std::vector<__nv_bfloat16> imga;
@@ -614,23 +591,6 @@ int dcb_load_weights(dcb_engine* e, const dcb_tensor* tensors, int32_t n) {
     const float* b1 = tm.get(P1 + "/layer/filter_dense_layer/bias", {ff}, &rc); if (rc) return rc;
     const float* w2 = tm.get(P1 + "/layer/output_dense_layer/kernel", {ff, kD}, &rc); if (rc) return rc;
     const float* b2 = tm.get(P1 + "/layer/output_dense_layer/bias", {kD}, &rc); if (rc) return rc;
-    {
-      std::vector<__nv_bfloat16> img;
-      img.reserve((size_t)ff * kDP * 2);
-      for (int ch = 0; ch < ff / kFFChunk; ++ch) {
-        auto p1 = pack_b(kDP, kFFChunk, [&](int k, int nn) {
-          return k < kD ? w1[(size_t)k * ff + ch * kFFChunk + nn] : 0.f;
-        });
-        auto p2 = pack_b(kFFChunk, kDP, [&](int k, int nn) {
-          return nn < kD ? w2[(size_t)(ch * kFFChunk + k) * kD + nn] * alpha1 : 0.f;
-        });
-        img.insert(img.end(), p1.begin(), p1.end());
-        img.insert(img.end(), p2.begin(), p2.end());
-      }
-      __nv_bfloat16* dptr = nullptr;
-      if ((rc = upload(e, &dptr, img))) return rc;
-      ld.wffn = reinterpret_cast<uint8_t*>(dptr);
-    }
     {
       // CTA-pair image: rank r holds hidden units c*128 + r*64 + [0,64) of W1 and, for each 144-wide
       // N chunk j of W2, output rows j*144 + r*72 + [0,72)
@@ -966,7 +926,7 @@ static int submit_impl(dcb_engine* e, const float* rows, const uint8_t* packed, 
       hp.M = M; hp.L = L; hp.Lw = Lw;
       return hp;
     };
-    const bool use_stack = e->stack && e->fuse_qa && e->ffn_pair && e->fuse_oproj && e->fuse_embed && !e->debug &&
+    const bool use_stack = e->stack && e->fuse_qa && e->fuse_oproj && e->fuse_embed && !e->debug &&
                            (Lw == kTileM || (Lw == 2 * kTileM && L > kTileM)) &&
                            c.attn_win_size > 0 && c.attn_win_size <= 16 && c.num_hidden_layers <= kMaxLayers;
     {
@@ -1029,15 +989,14 @@ static int submit_impl(dcb_engine* e, const float* rows, const uint8_t* packed, 
         --launches;   // one launch instead of two (3 per layer are added below)
       } else {
         pbegin(2);
-        if (e->qkv2) launch_qkv2(e->d_xb, ld.wqkv2, T, e->d_embqkv, st);
-        else launch_gemm_qkv(e->d_xb, ld.wqkv, T, e->d_embqkv, st);
+        launch_gemm_qkv(e->d_xb, ld.wqkv, T, e->d_embqkv, st);
         pend();
         pbegin(3);
         launch_attention(e->d_embqkv, e->d_att, L, Lw, c.attn_win_size, bw, st);
         pend();
       }
       // attention out-proj + FFN: fused into one CTA-pair kernel unless debugging the intermediate
-      const bool fused = e->ffn_pair && e->fuse_oproj && !e->debug;
+      const bool fused = e->fuse_oproj && !e->debug;
       RowEpi ef{};
       ef.x = e->d_x; ef.xb = last ? nullptr : e->d_xb; ef.bias = ld.b2; ef.pe = nullptr;
       ef.ln_g = (c.rezero || last) ? nullptr : e->layers[n_ + 1].ln_g[0];
@@ -1059,10 +1018,8 @@ static int submit_impl(dcb_engine* e, const float* rows, const uint8_t* packed, 
       if (fused)
         launch_ffn_pair(e->d_att, ld.wffn2, ld.b1, c.filter_size, T, ef, st, ld.wo2,
                         c.rezero ? nullptr : ld.ln_g[1], c.rezero ? nullptr : ld.ln_b[1]);
-      else if (e->ffn_pair)
-        launch_ffn_pair(e->d_xb, ld.wffn2, ld.b1, c.filter_size, T, ef, st);
       else
-        launch_ffn(e->d_xb, ld.wffn, ld.b1, c.filter_size, T, ef, st);
+        launch_ffn_pair(e->d_xb, ld.wffn2, ld.b1, c.filter_size, T, ef, st);
       pend();
       if (e->profile) e->prof_ffn_tokens += (long long)bw * L;   // valid tokens (layout padding is not algorithmic work)
       if (!fused) snap();

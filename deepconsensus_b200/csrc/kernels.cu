@@ -6,11 +6,18 @@
 //   gemm_kernel         persistent, warp-specialised tcgen05 GEMM: bulk-copy (TMA) producer
 //                       warp, single-thread UMMA issuer, 4 epilogue warps reading TMEM.
 //                       Used for the condenser (+pos-enc), fused QKV, attention out-proj.
+//   embed_condense_kernel  embedding + condenser GEMM in one pass (CTA pairs); the bf16
+//                       embedding never goes to HBM
+//   ffn_pair_kernel     fused FFN on CTA pairs: relu(x W1 + b1) W2 + b2 with the [128 x 2048]
+//                       hidden activation living only in TMEM/SMEM (ffn_layer.py:83-86),
+//                       optionally behind the attention out-projection
 //   band_attention_kernel  banded multi-head softmax attention (attention_layer.py:198-214)
-//   ffn_kernel          fused FFN: relu(x W1 + b1) W2 + b2 with the [128 x 2048] hidden
-//                       activation living only in TMEM/SMEM (ffn_layer.py:83-86)
+//   qkv_attn_pair_kernel   fused QKV projection + banded attention on window-aligned tiles
+//   stack_pair_kernel   the whole encoder stack (+ head) in one launch (stack_kernel.cuh)
 //   head_kernel         final LayerNorm -> fc1 -> softmax -> argmax -> Phred -> ASCII
 //                       (encoder_stack.py:197, networks.py:342,238, quick_inference.py:377-414)
+//   unpack_rows_kernel  packed rows -> float32 [B, R, L] rows
+//   stitch_kernel       per-read window concatenation + gap compaction (stitch_utils.py:51-98)
 #include "kernels.h"
 
 #include <cuda_bf16.h>
@@ -1017,502 +1024,7 @@ size_t embed_condense_smem_bytes(int R, int echunks, int table_elems, int packed
 }
 
 // =====================================================================================
-// fused q/k/v projection, two tiles per weight pass
-// =====================================================================================
-// The QKV projection re-reads 498 KB of weights per 128-token tile, and an SM ingests only about
-// 30-50 B/cycle from L2, so the per-tile weight stream (not the 7.8 k cycles of UMMA work) sets the
-// pace.  This kernel therefore keeps TWO x tiles resident in shared memory and runs both against
-// every weight stage (halving the weight bytes per token), processes the 864 output columns in 9
-// groups of 96, and double-buffers the accumulators in TMEM (2 x [2 tiles x 96 cols]) so the
-// epilogue of group g (TMEM -> bf16 -> qkv operand image) overlaps the UMMAs of group g+1.
-struct Qkv2Cfg {
-  static constexpr int kGroupN = 96;
-  static constexpr int kGroups = kQKVN / kGroupN;                    // 9
-  static constexpr int kABytes = (kDP / 8) * kTileM * 16;            // 73728 per tile
-  static constexpr int kStageK = 6;
-  static constexpr int kStages = (kDP / 16) / kStageK;               // 3 stages per group
-  static constexpr int kStageBytes = kStageK * 2 * kGroupN * 16;     // 18432
-  static constexpr int kSlots = 3;
-  static constexpr int kGroupBytes = kStages * kStageBytes;          // 55296
-  static constexpr int kOffA0 = 0;
-  static constexpr int kOffA1 = kABytes;
-  static constexpr int kOffRing = 2 * kABytes;
-  static constexpr int kOffBars = kOffRing + kSlots * kStageBytes;
-  static constexpr int kSmemBytes = kOffBars + 256;
-  static constexpr int kTmemCols = 512;
-  static constexpr int kThreads = 320;   // producer, UMMA issuer, 8 epilogue warps (4 per tile)
-};
-
-__global__ void __launch_bounds__(Qkv2Cfg::kThreads, 1)
-qkv2_kernel(const __nv_bfloat16* __restrict__ a_img, const uint8_t* __restrict__ b_img, int ntiles,
-            __nv_bfloat16* __restrict__ out_img) {
-  using C = Qkv2Cfg;
-  extern __shared__ __align__(1024) uint8_t smem[];
-  uint8_t* sA[2] = {smem + C::kOffA0, smem + C::kOffA1};
-  uint8_t* sRing = smem + C::kOffRing;
-  uint64_t* bars = reinterpret_cast<uint64_t*>(smem + C::kOffBars);
-  uint64_t* full = bars;                  // [kSlots]
-  uint64_t* empty = bars + C::kSlots;     // [kSlots]
-  uint64_t* a_full = bars + 2 * C::kSlots;
-  uint64_t* a_empty = a_full + 1;
-  uint64_t* acc_full = a_full + 2;        // [2]
-  uint64_t* acc_empty = a_full + 4;       // [2]
-  uint32_t* tmem_holder = reinterpret_cast<uint32_t*>(a_full + 6);
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int npairs = (ntiles + 1) >> 1;
-
-  if (threadIdx.x == 0) {
-    for (int i = 0; i < C::kSlots; ++i) { mbar_init(&full[i], 1); mbar_init(&empty[i], 1); }
-    mbar_init(a_full, 1);
-    mbar_init(a_empty, 1);
-    mbar_init(&acc_full[0], 1);
-    mbar_init(&acc_full[1], 1);
-    mbar_init(&acc_empty[0], 256);
-    mbar_init(&acc_empty[1], 256);
-    mbar_fence_init();
-  }
-  if (warp == 1) tmem_alloc(tmem_holder, C::kTmemCols);
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_holder;
-
-  if (warp == 0) {
-    if (lane == 0) {
-      uint32_t slot = 0, phase = 0, it = 0;
-      for (int p = blockIdx.x; p < npairs; p += gridDim.x, ++it) {
-        mbar_wait(a_empty, (it & 1) ^ 1);
-        mbar_arrive_expect_tx(a_full, 2 * C::kABytes);
-        const int t0 = 2 * p, t1 = min(2 * p + 1, ntiles - 1);
-        bulk_g2s(sA[0], reinterpret_cast<const uint8_t*>(a_img) + (size_t)t0 * C::kABytes, C::kABytes, a_full);
-        bulk_g2s(sA[1], reinterpret_cast<const uint8_t*>(a_img) + (size_t)t1 * C::kABytes, C::kABytes, a_full);
-        for (int g = 0; g < C::kGroups; ++g)
-          for (int s = 0; s < C::kStages; ++s) {
-            mbar_wait(&empty[slot], phase ^ 1);
-            mbar_arrive_expect_tx(&full[slot], C::kStageBytes);
-            bulk_g2s(sRing + slot * C::kStageBytes, b_img + (size_t)g * C::kGroupBytes + s * C::kStageBytes,
-                     C::kStageBytes, &full[slot]);
-            if (++slot == C::kSlots) { slot = 0; phase ^= 1; }
-          }
-      }
-    }
-  } else if (warp == 1) {
-    if (lane == 0) {
-      constexpr uint32_t idesc = make_idesc_bf16(kTileM, C::kGroupN);
-      const uint32_t a_addr[2] = {smem_u32(sA[0]), smem_u32(sA[1])};
-      uint32_t slot = 0, phase = 0, it = 0, gi = 0;
-      for (int p = blockIdx.x; p < npairs; p += gridDim.x, ++it) {
-        mbar_wait(a_full, it & 1);
-        tc_fence_after();
-        for (int g = 0; g < C::kGroups; ++g, ++gi) {
-          const uint32_t buf = gi & 1;
-          mbar_wait(&acc_empty[buf], ((gi >> 1) & 1) ^ 1);
-          tc_fence_after();
-          for (int s = 0; s < C::kStages; ++s) {
-            mbar_wait(&full[slot], phase);
-            tc_fence_after();
-            const uint32_t sb = smem_u32(sRing + slot * C::kStageBytes);
-#pragma unroll
-            for (int kk = 0; kk < C::kStageK; ++kk) {
-              const int kstep = s * C::kStageK + kk;
-              const uint64_t bdesc = make_kc16_desc(sb + kk * (2 * C::kGroupN * 16), C::kGroupN * 16, 128);
-#pragma unroll
-              for (int t = 0; t < 2; ++t) {
-                const uint64_t adesc = make_kc16_desc(a_addr[t] + kstep * 4096, kTileM * 16, 128);
-                umma_bf16_ss(tmem_base + buf * (2 * C::kGroupN) + t * C::kGroupN, adesc, bdesc, idesc, kstep != 0);
-              }
-            }
-            umma_commit(&empty[slot]);
-            if (++slot == C::kSlots) { slot = 0; phase ^= 1; }
-          }
-          umma_commit(&acc_full[buf]);
-        }
-        umma_commit(a_empty);
-      }
-    }
-  } else {
-    const int q = warp & 3;
-    const int t = (warp - 2) >> 2;          // which tile of the pair
-    const int r = q * 32 + lane;
-    const uint32_t tmem_row = tmem_base + ((uint32_t)(q * 32) << 16);
-    uint32_t gi = 0;
-    for (int p = blockIdx.x; p < npairs; p += gridDim.x) {
-      const int tile = 2 * p + t;
-      const bool valid = tile < ntiles;
-      uint4* orow = reinterpret_cast<uint4*>(out_img + (size_t)(valid ? tile : 0) * kTileM * kQKVN) + r;
-      for (int g = 0; g < C::kGroups; ++g, ++gi) {
-        const uint32_t buf = gi & 1;
-        mbar_wait(&acc_full[buf], (gi >> 1) & 1);
-        tc_fence_after();
-        uint32_t acc[C::kGroupN / 16][16];
-#pragma unroll
-        for (int cb = 0; cb < C::kGroupN / 16; ++cb)
-          tmem_ld16(tmem_row + buf * (2 * C::kGroupN) + t * C::kGroupN + cb * 16, acc[cb]);
-        tmem_ld_wait();
-        tc_fence_before();
-        mbar_arrive(&acc_empty[buf]);
-        if (valid) {
-#pragma unroll
-          for (int cb = 0; cb < C::kGroupN / 16; ++cb) {
-            const int kc = (g * C::kGroupN + cb * 16) / 8;
-            float v[16];
-#pragma unroll
-            for (int i = 0; i < 16; ++i) v[i] = __uint_as_float(acc[cb][i]);
-            orow[(size_t)kc * kTileM] = make_uint4(pack_bf16x2(v[0], v[1]), pack_bf16x2(v[2], v[3]),
-                                                   pack_bf16x2(v[4], v[5]), pack_bf16x2(v[6], v[7]));
-            orow[(size_t)(kc + 1) * kTileM] =
-                make_uint4(pack_bf16x2(v[8], v[9]), pack_bf16x2(v[10], v[11]),
-                           pack_bf16x2(v[12], v[13]), pack_bf16x2(v[14], v[15]));
-          }
-        }
-      }
-    }
-  }
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 1) {
-    tc_fence_after();
-    tmem_dealloc(tmem_base, C::kTmemCols);
-  }
-}
-
-// =====================================================================================
-// fused FFN
-// =====================================================================================
-struct FfnCfg {
-  static constexpr int kABytes = (kDP / 8) * kTileM * 16;            // 73728: x operand tile
-  static constexpr int kHBytes = (kFFChunk / 8) * kTileM * 16;       // 32768: one hidden chunk
-  static constexpr int kSlotBytes = 24576;
-  static constexpr int kSlots = 3;
-  static constexpr int kW1StageK = 6;                                // k-steps per W1 stage
-  static constexpr int kW1StageBytes = kW1StageK * 2 * kFFChunk * 16;  // 24576
-  static constexpr int kW1Stages = (kDP / 16) / kW1StageK;           // 3
-  static constexpr int kW2StageK = 2;                                // k-steps per W2 stage
-  static constexpr int kW2StageBytes = kW2StageK * 2 * kDP * 16;     // 18432
-  static constexpr int kW2Stages = (kFFChunk / 16) / kW2StageK;      // 4
-  static constexpr int kW1ChunkBytes = kW1Stages * kW1StageBytes;    // 73728
-  static constexpr int kW2ChunkBytes = kW2Stages * kW2StageBytes;    // 73728
-  static constexpr int kTmemY = 0;
-  static constexpr int kTmemH = kDP;                                 // 288
-  static constexpr int kTmemCols = 512;
-  static constexpr int kMaxFF = 2048;
-  static constexpr int kOffA = 0;
-  static constexpr int kOffH = kABytes;
-  static constexpr int kOffRing = kOffH + 2 * kHBytes;
-  static constexpr int kOffB1 = kOffRing + kSlots * kSlotBytes;
-  static constexpr int kOffBars = kOffB1 + kMaxFF * 4;
-  static constexpr int kSmemBytes = kOffBars + 256;
-};
-static_assert(FfnCfg::kSmemBytes <= 232448, "FFN shared memory budget");
-static_assert(FfnCfg::kW1StageBytes <= FfnCfg::kSlotBytes && FfnCfg::kW2StageBytes <= FfnCfg::kSlotBytes, "slot");
-
-// w_img: per ff-chunk c: [W1 chunk image 73728 B][W2 chunk image 73728 B].
-//
-// CS = thread-block cluster size.  The CS CTAs of a cluster walk their tiles in lock step and
-// share every weight stage: CTA `rank` fetches 1/CS of the stage and multicasts it into the
-// same ring slot of all CS CTAs (cp.async.bulk ... .multicast::cluster), which divides the
-// L2 -> SM weight traffic by CS (an un-clustered CTA streams all 2.36 MB of layer weights per
-// 128-token tile, which saturates L2 bandwidth long before the tensor pipe).  A ring slot is
-// recycled when the MMAs of ALL CS CTAs that read it have completed (multicast tcgen05.commit
-// onto every CTA's `empty` barrier, count = CS).
-//
-// Four warpgroups: WG0 = {bulk-copy producer, UMMA issuer (+TMEM alloc), 2 idle warps};
-// WG1+WG2 = hidden-chunk epilogue (two warps share each TMEM lane quarter and split the chunk's
-// columns, halving the G1 -> epilogue -> G1 dependency chain); WG3 = row epilogue of the finished
-// tile, which thereby overlaps the next tile's GEMMs (its residual loads are software-prefetched).
-// setmaxnreg moves registers from WG0-2 to WG3, whose fully unrolled prefetching loop needs ~200.
-constexpr int kFfnThreads = 512;
-
-// Optional cycle trace (build with -DDCB_TRACE): per CTA, cycles the MMA thread and one
-// hidden-epilogue warp spend in each wait.  Read back with dcb_debug_trace().
-
-
-template <int CS>
-__global__ void __launch_bounds__(kFfnThreads, 1)
-ffn_kernel(const __nv_bfloat16* __restrict__ a_img, const uint8_t* __restrict__ w_img,
-           const float* __restrict__ b1, int ff, int ntiles, RowEpi epi) {
-  using C = FfnCfg;
-  extern __shared__ __align__(1024) uint8_t smem[];
-  uint8_t* sA = smem + C::kOffA;
-  uint8_t* sH = smem + C::kOffH;
-  uint8_t* sRing = smem + C::kOffRing;
-  float* sB1 = reinterpret_cast<float*>(smem + C::kOffB1);
-  uint64_t* bars = reinterpret_cast<uint64_t*>(smem + C::kOffBars);
-  uint64_t* full = bars;                   // [kSlots]
-  uint64_t* empty = bars + C::kSlots;      // [kSlots]
-  uint64_t* a_full = bars + 2 * C::kSlots;
-  uint64_t* a_empty = a_full + 1;
-  uint64_t* h_full = a_full + 2;           // MMA -> epilogue: hidden chunk accumulator ready
-  uint64_t* h_free = a_full + 3;           // epilogue -> MMA: hidden TMEM columns drained
-  uint64_t* hs_full = a_full + 4;          // [2] epilogue -> MMA: bf16 hidden chunk in smem
-  uint64_t* hs_free = a_full + 6;          // [2] MMA -> epilogue: smem hidden chunk consumed
-  uint64_t* y_full = a_full + 8;
-  uint64_t* y_empty = a_full + 9;
-  uint32_t* tmem_holder = reinterpret_cast<uint32_t*>(a_full + 10);
-
-  const int warp = threadIdx.x >> 5;
-  const int lane = threadIdx.x & 31;
-  const int nchunks = ff / kFFChunk;
-  const uint32_t rank = CS > 1 ? cluster_ctarank() : 0u;
-  constexpr uint16_t kMask = (uint16_t)((1u << CS) - 1u);
-  // every CTA of a cluster runs the same number of rounds; a CTA whose tile index falls past the
-  // end recomputes the last tile and drops the result, so the shared weight pipeline stays uniform
-  const int rounds = (ntiles + (int)gridDim.x - 1) / (int)gridDim.x;
-
-  if (threadIdx.x == 0) {
-    for (int i = 0; i < C::kSlots; ++i) {
-      mbar_init(&full[i], 1);
-      mbar_init(&empty[i], CS);
-    }
-    mbar_init(a_full, 1);
-    mbar_init(a_empty, 1);
-    mbar_init(h_full, 1);
-    mbar_init(h_free, 256);
-    mbar_init(&hs_full[0], 256);
-    mbar_init(&hs_full[1], 256);
-    mbar_init(&hs_free[0], 1);
-    mbar_init(&hs_free[1], 1);
-    mbar_init(y_full, 1);
-    mbar_init(y_empty, 128);
-    mbar_fence_init();
-  }
-  for (int i = threadIdx.x; i < ff; i += blockDim.x) sB1[i] = b1[i];
-  if (warp == 1) tmem_alloc(tmem_holder, C::kTmemCols);
-  tc_fence_before();
-  __syncthreads();
-  if (CS > 1) cluster_sync_all();   // peers' barriers are initialised before any multicast lands
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_holder;
-
-  if (warp < 4) {
-   setmaxnreg_dec<64>();
-   if (warp == 0) {
-    // ------------------------------------------------------------- producer
-    if (lane == 0) {
-      uint32_t slot = 0, phase = 0;
-      auto push = [&](const uint8_t* src, uint32_t bytes) {
-        mbar_wait(&empty[slot], phase ^ 1);
-        mbar_arrive_expect_tx(&full[slot], bytes);
-        if (CS == 1) {
-          bulk_g2s(sRing + slot * C::kSlotBytes, src, bytes, &full[slot]);
-        } else {
-          const uint32_t part = bytes / CS;
-          bulk_g2s_multicast(sRing + slot * C::kSlotBytes + rank * part, src + rank * part, part,
-                             &full[slot], kMask);
-        }
-        if (++slot == C::kSlots) { slot = 0; phase ^= 1; }
-      };
-      auto push_w1 = [&](int c) {
-        const uint8_t* src = w_img + (size_t)c * (C::kW1ChunkBytes + C::kW2ChunkBytes);
-        for (int s = 0; s < C::kW1Stages; ++s) push(src + s * C::kW1StageBytes, C::kW1StageBytes);
-      };
-      auto push_w2 = [&](int c) {
-        const uint8_t* src =
-            w_img + (size_t)c * (C::kW1ChunkBytes + C::kW2ChunkBytes) + C::kW1ChunkBytes;
-        for (int s = 0; s < C::kW2Stages; ++s) push(src + s * C::kW2StageBytes, C::kW2StageBytes);
-      };
-      for (int ti = 0; ti < rounds; ++ti) {
-        const int tile = min(ti * (int)gridDim.x + (int)blockIdx.x, ntiles - 1);
-        mbar_wait(a_empty, (ti & 1) ^ 1);
-        mbar_arrive_expect_tx(a_full, C::kABytes);
-        bulk_g2s(sA, reinterpret_cast<const uint8_t*>(a_img) + (size_t)tile * C::kABytes,
-                 C::kABytes, a_full);
-        // same order as the MMA warp consumes: W1(0), then W1(c+1), W2(c) ...
-        push_w1(0);
-        for (int c = 0; c < nchunks; ++c) {
-          if (c + 1 < nchunks) push_w1(c + 1);
-          push_w2(c);
-        }
-      }
-    }
-  } else if (warp == 1) {
-    // ------------------------------------------------------------- MMA issuer
-    if (lane == 0) {
-      constexpr uint32_t idesc_h = make_idesc_bf16(kTileM, kFFChunk);
-      constexpr uint32_t idesc_y = make_idesc_bf16(kTileM, kNC);
-      const uint32_t a_addr = smem_u32(sA);
-      uint32_t slot = 0, phase = 0, n = 0;  // n: global hidden-chunk counter
-      long long t_hfree = 0, t_full = 0, t_hsfull = 0, t_issue = 0, t_afull = 0, t_yempty = 0, t_oproj = 0, t_a2full = 0;
-      const long long t_begin = clock64();
-      auto release = [&](uint64_t* bar) {
-        if (CS == 1) umma_commit(bar); else umma_commit_multicast(bar, kMask);
-      };
-      auto gemm1 = [&](uint32_t nn) {
-        // H[128 x 128] = X[128 x 288] * W1chunk^T
-        TRACE_T0();
-        mbar_wait(h_free, (nn & 1) ^ 1);
-        TRACE_ADD(t_hfree);
-        tc_fence_after();
-        for (int s = 0; s < C::kW1Stages; ++s) {
-          mbar_wait(&full[slot], phase);
-          TRACE_ADD(t_full);
-          tc_fence_after();
-          const uint32_t sb = smem_u32(sRing + slot * C::kSlotBytes);
-#pragma unroll
-          for (int kk = 0; kk < C::kW1StageK; ++kk) {
-            const int kstep = s * C::kW1StageK + kk;
-            const uint64_t adesc = make_kc16_desc(a_addr + kstep * 4096, kTileM * 16, 128);
-            const uint64_t bdesc = make_kc16_desc(sb + kk * (2 * kFFChunk * 16), kFFChunk * 16, 128);
-            umma_bf16_ss(tmem_base + C::kTmemH, adesc, bdesc, idesc_h, kstep != 0);
-          }
-          release(&empty[slot]);
-          if (++slot == C::kSlots) { slot = 0; phase ^= 1; }
-          TRACE_ADD(t_issue);
-        }
-        umma_commit(h_full);
-      };
-      auto gemm2 = [&](uint32_t nn, int c) {
-        // Y[128 x 288] += Hc[128 x 128] * W2chunk^T
-        const uint32_t b = nn & 1;
-        TRACE_T0();
-        mbar_wait(&hs_full[b], (nn >> 1) & 1);
-        TRACE_ADD(t_hsfull);
-        tc_fence_after();
-        const uint32_t h_addr = smem_u32(sH + b * C::kHBytes);
-        for (int s = 0; s < C::kW2Stages; ++s) {
-          mbar_wait(&full[slot], phase);
-          TRACE_ADD(t_full);
-          tc_fence_after();
-          const uint32_t sb = smem_u32(sRing + slot * C::kSlotBytes);
-#pragma unroll
-          for (int kk = 0; kk < C::kW2StageK; ++kk) {
-            const int kstep = s * C::kW2StageK + kk;
-            const uint64_t adesc = make_kc16_desc(h_addr + kstep * 4096, kTileM * 16, 128);
-#pragma unroll
-            for (int j = 0; j < 2; ++j) {
-              const uint64_t bdesc =
-                  make_kc16_desc(sb + kk * (2 * kDP * 16) + j * kNC * 16, kDP * 16, 128);
-              umma_bf16_ss(tmem_base + C::kTmemY + j * kNC, adesc, bdesc, idesc_y, (c | kstep) != 0);
-            }
-          }
-          release(&empty[slot]);
-          if (++slot == C::kSlots) { slot = 0; phase ^= 1; }
-        }
-        umma_commit(&hs_free[b]);
-      };
-      for (int ti = 0; ti < rounds; ++ti) {
-        { TRACE_T0(); mbar_wait(a_full, ti & 1); TRACE_ADD(t_afull); }
-        tc_fence_after();
-        gemm1(n);
-        for (int c = 0; c < nchunks; ++c) {
-          if (c + 1 < nchunks) {
-            gemm1(n + c + 1);
-          } else {
-            umma_commit(a_empty);          // all GEMM1s of this tile issued: x tile reusable
-          }
-          if (c == 0) {
-            TRACE_T0();
-            mbar_wait(y_empty, (ti & 1) ^ 1);  // previous tile's Y drained by the epilogue
-            TRACE_ADD(t_yempty);
-            tc_fence_after();
-          }
-          gemm2(n + c, c);
-        }
-        umma_commit(y_full);
-        n += nchunks;
-      }
-#ifdef DCB_TRACE
-      if (blockIdx.x < 256) {
-        unsigned long long* tr = g_ffn_trace + blockIdx.x * 16;
-        tr[0] = clock64() - t_begin; tr[1] = t_hfree; tr[2] = t_full; tr[3] = t_hsfull;
-        tr[4] = t_issue; tr[5] = t_afull; tr[6] = t_yempty; tr[7] = t_a2full; tr[15] = t_oproj;
-      }
-#endif
-    }
-   }
-  } else {
-    // ------------------------------------------------------------- epilogue warps
-    const int q = warp & 3;            // TMEM lane quarter
-    const int r = q * 32 + lane;
-    const uint32_t tmem_row = tmem_base + ((uint32_t)(q * 32) << 16);
-    if (warp < 12) {
-      setmaxnreg_dec<96>();
-      // hidden-chunk epilogue: TMEM -> +b1, relu -> bf16 -> smem operand of GEMM2
-      const int half = (warp - 4) >> 2;  // which 64 columns of the hidden chunk
-      uint32_t n = 0;
-      long long t_hfull = 0, t_hsfree = 0, t_body = 0;
-      for (int ti = 0; ti < rounds; ++ti) {
-        for (int c = 0; c < nchunks; ++c, ++n) {
-          const uint32_t b = n & 1;
-          TRACE_T0();
-          mbar_wait(h_full, n & 1);
-          TRACE_ADD(t_hfull);
-          tc_fence_after();
-          mbar_wait(&hs_free[b], ((n >> 1) & 1) ^ 1);
-          TRACE_ADD(t_hsfree);
-          uint4* hrow = reinterpret_cast<uint4*>(sH + b * C::kHBytes) + r;
-          const float* bias = sB1 + c * kFFChunk;
-#pragma unroll
-          for (int cc = 0; cc < kFFChunk / 32; ++cc) {
-            const int cb = half * (kFFChunk / 32) + cc;
-            uint32_t acc[16];
-            tmem_ld16(tmem_row + C::kTmemH + cb * 16, acc);
-            tmem_ld_wait();
-            float v[16];
-#pragma unroll
-            for (int i = 0; i < 16; ++i) v[i] = fmaxf(__uint_as_float(acc[i]) + bias[cb * 16 + i], 0.f);
-            hrow[(size_t)(cb * 2) * kTileM] = make_uint4(pack_bf16x2(v[0], v[1]), pack_bf16x2(v[2], v[3]),
-                                                         pack_bf16x2(v[4], v[5]), pack_bf16x2(v[6], v[7]));
-            hrow[(size_t)(cb * 2 + 1) * kTileM] =
-                make_uint4(pack_bf16x2(v[8], v[9]), pack_bf16x2(v[10], v[11]),
-                           pack_bf16x2(v[12], v[13]), pack_bf16x2(v[14], v[15]));
-          }
-          tc_fence_before();
-          mbar_arrive(h_free);
-          fence_proxy_async_smem();
-          mbar_arrive(&hs_full[b]);
-          TRACE_ADD(t_body);
-        }
-      }
-#ifdef DCB_TRACE
-      if (warp == 4 && lane == 0 && blockIdx.x < 256) {
-        unsigned long long* tr = g_ffn_trace + blockIdx.x * 16;
-        tr[8] = t_hfull; tr[9] = t_hsfree; tr[10] = t_body;
-      }
-#endif
-    } else {
-      setmaxnreg_inc<216>();
-      // row epilogue of each finished tile (overlaps the next tile's GEMMs)
-      long long t_yfull = 0, t_row = 0;
-      for (int ti = 0; ti < rounds; ++ti) {
-        const int tile_raw = ti * (int)gridDim.x + (int)blockIdx.x;
-        const bool valid = tile_raw < ntiles;
-        RowPrefetch pf;
-        if (valid) row_prefetch_start(epi, tile_raw, r, pf);
-        TRACE_T0();
-        mbar_wait(y_full, ti & 1);
-        TRACE_ADD(t_yfull);
-        tc_fence_after();
-        if (valid) {
-          const RowStats st = row_epilogue_pass1(epi, tmem_row + C::kTmemY, tile_raw, r, pf);
-          tc_fence_before();
-          mbar_arrive(y_empty);
-          if (epi.ln_g && epi.xb) row_epilogue_pass2<false>(epi, tile_raw, r, st.mean, st.rstd);
-        } else {
-          tc_fence_before();
-          mbar_arrive(y_empty);
-        }
-        TRACE_ADD(t_row);
-      }
-#ifdef DCB_TRACE
-      if (warp == 12 && lane == 0 && blockIdx.x < 256) {
-        unsigned long long* tr = g_ffn_trace + blockIdx.x * 16;
-        tr[11] = t_yfull; tr[12] = t_row;
-      }
-#endif
-    }
-  }
-  tc_fence_before();
-  __syncthreads();
-  if (CS > 1) cluster_sync_all();   // no CTA exits while a peer may still multicast into it
-  if (warp == 1) {
-    tc_fence_after();
-    tmem_dealloc(tmem_base, C::kTmemCols);
-  }
-}
-
-// =====================================================================================
-// fused FFN, CTA-pair version (tcgen05 cta_group::2)
+// fused FFN on CTA pairs (tcgen05 cta_group::2)
 // =====================================================================================
 // Two CTAs (a cluster of 2 = one TPC's SM pair) process two 128-token tiles together with M=256
 // UMMAs issued by the leader (cluster rank 0).  Each CTA keeps its own x tile, hidden chunk and
@@ -1561,6 +1073,13 @@ struct Ffn2Cfg {
 };
 static_assert(Ffn2Cfg::kSmemBytes <= 232448, "FFN pair shared memory budget");
 static_assert(Ffn2Cfg::kW1Stages * Ffn2Cfg::kW1StageK == kDP / 16 && Ffn2Cfg::kW2Stages * Ffn2Cfg::kW2StageK == kFFChunk / 16, "stages");
+
+// Four warpgroups: WG0 = {bulk-copy producer, two UMMA issuers (leader) or the relay thread (peer), 1 idle warp};
+// WG1+WG2 = hidden-chunk epilogue (two warps share each TMEM lane quarter and split the chunk's columns, halving the
+// G1 -> epilogue -> G1 dependency chain); WG3 = row epilogue of the finished tile, which thereby overlaps the next
+// tile's GEMMs (its residual loads are software-prefetched).  setmaxnreg moves registers from WG0-2 to WG3, whose
+// fully unrolled prefetching loop needs ~200.
+constexpr int kFfnThreads = 512;
 
 // kFuse: the attention output projection (attention_layer.py:218) + its residual / pre-norm
 // (encoder_stack.py:72-93) run in front of the FFN on the same tile: a_img is then the attention
@@ -2870,19 +2389,11 @@ cudaError_t kernels_init() {
   if (e != cudaSuccess) return e;
   e = cudaFuncSetAttribute(stack_pair_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, StackCfg::kSmemBytes);
   if (e != cudaSuccess) return e;
-  e = cudaFuncSetAttribute(ffn_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, FfnCfg::kSmemBytes);
-  if (e != cudaSuccess) return e;
-  e = cudaFuncSetAttribute(ffn_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, FfnCfg::kSmemBytes);
-  if (e != cudaSuccess) return e;
-  e = cudaFuncSetAttribute(ffn_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, FfnCfg::kSmemBytes);
-  if (e != cudaSuccess) return e;
   e = cudaFuncSetAttribute(qkv_attn_pair_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, QaCfg::kSmemBytes);
   if (e != cudaSuccess) return e;
   e = cudaFuncSetAttribute(qkv_attn_pair_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, QaCfg::kSmemBytes);
   if (e != cudaSuccess) return e;
   e = cudaFuncSetAttribute(embed_condense_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 225 * 1024);   // + 2 KB static
-  if (e != cudaSuccess) return e;
-  e = cudaFuncSetAttribute(qkv2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, Qkv2Cfg::kSmemBytes);
   if (e != cudaSuccess) return e;
   e = cudaFuncSetAttribute(embed_rows_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024);
   if (e != cudaSuccess) return e;
@@ -2953,13 +2464,6 @@ void launch_unpack_rows(const uint8_t* packed, const PackedLayout& pl, int nwind
   if (nwindows > 0) unpack_rows_kernel<<<nwindows, 256, 0, st>>>(packed, pl, nwindows, rows);
 }
 
-void launch_qkv2(const __nv_bfloat16* a_img, const uint8_t* b_img, int ntiles, __nv_bfloat16* qkv_img,
-                 cudaStream_t st) {
-  const int npairs = (ntiles + 1) / 2;
-  const int grid = npairs < num_sms() ? npairs : num_sms();
-  qkv2_kernel<<<grid, Qkv2Cfg::kThreads, Qkv2Cfg::kSmemBytes, st>>>(a_img, b_img, ntiles, qkv_img);
-}
-
 void launch_qkv_attn(const __nv_bfloat16* a_img, const uint8_t* w_img, int ntiles, int L, int win,
                      __nv_bfloat16* att, cudaStream_t st) {
   static int max_pairs = 0;
@@ -3007,37 +2511,6 @@ void launch_attention(const __nv_bfloat16* qkv, __nv_bfloat16* att, int L, int L
   band_attention_kernel<<<nwindows * 2, 128, smem, st>>>(qkv, att, L, Lw, win, nwindows);
 }
 
-static int g_ffn_cluster = 0;
-
-template <int CS>
-static void launch_ffn_cs(const __nv_bfloat16* a_img, const uint8_t* w_img, const float* b1, int ff,
-                          int ntiles, const RowEpi& epi, cudaStream_t st) {
-  cudaLaunchConfig_t cfg{};
-  cfg.blockDim = dim3(kFfnThreads);
-  cfg.dynamicSmemBytes = FfnCfg::kSmemBytes;
-  cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = CS;
-  attr[0].val.clusterDim.y = 1;
-  attr[0].val.clusterDim.z = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = 1;
-  // persistent grid = as many clusters as can be co-resident (GPC sizes strand a few SMs for CS=4)
-  static int max_clusters = 0;
-  if (!max_clusters) {
-    cfg.gridDim = dim3(num_sms() / CS * CS);
-    int nc = 0;
-    if (cudaOccupancyMaxActiveClusters(&nc, ffn_kernel<CS>, &cfg) != cudaSuccess || nc <= 0) nc = num_sms() / CS;
-    max_clusters = nc;
-    if (dev_env("DCB_VERBOSE")) fprintf(stderr, "[dcb200] ffn cluster size %d: %d co-resident clusters\n", CS, nc);
-  }
-  int clusters = (ntiles + CS - 1) / CS;
-  if (clusters > max_clusters) clusters = max_clusters;
-  cfg.gridDim = dim3(clusters * CS);
-  cudaLaunchKernelEx(&cfg, ffn_kernel<CS>, a_img, w_img, b1, ff, ntiles, epi);
-}
-
 void launch_ffn_pair(const __nv_bfloat16* a_img, const uint8_t* w2img, const float* b1, int ff, int ntiles,
                      const RowEpi& epi, cudaStream_t st, const uint8_t* wo2img, const float* mid_ln_g,
                      const float* mid_ln_b) {
@@ -3063,20 +2536,6 @@ void launch_ffn_pair(const __nv_bfloat16* a_img, const uint8_t* w2img, const flo
     cudaLaunchKernelEx(&cfg, ffn_pair_kernel<true>, a_img, w2img, b1, ff, ntiles, epi, stagger, wo2img, mid_ln_g, mid_ln_b);
   else
     cudaLaunchKernelEx(&cfg, ffn_pair_kernel<false>, a_img, w2img, b1, ff, ntiles, epi, stagger, wo2img, mid_ln_g, mid_ln_b);
-}
-
-void launch_ffn(const __nv_bfloat16* a_img, const uint8_t* w_img, const float* b1, int ff, int ntiles,
-                const RowEpi& epi, cudaStream_t st) {
-  if (!g_ffn_cluster) {
-    const char* env = dev_env("DCB_FFN_CLUSTER");
-    g_ffn_cluster = env ? atoi(env) : 1;   // measured: multicast does not pay here (smem-bound, not L2-bound)
-    if (g_ffn_cluster != 1 && g_ffn_cluster != 2 && g_ffn_cluster != 4) g_ffn_cluster = 1;
-  }
-  switch (g_ffn_cluster) {
-    case 1: launch_ffn_cs<1>(a_img, w_img, b1, ff, ntiles, epi, st); break;
-    case 2: launch_ffn_cs<2>(a_img, w_img, b1, ff, ntiles, epi, st); break;
-    default: launch_ffn_cs<4>(a_img, w_img, b1, ff, ntiles, epi, st); break;
-  }
 }
 
 int read_ffn_trace(unsigned long long* out, int n) {

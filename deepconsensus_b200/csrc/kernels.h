@@ -27,24 +27,19 @@ bool launch_embed_condense(const float* rows, const uint8_t* packed, const Packe
                            const EmbedRow* rowmeta, const __nv_bfloat16* tables, int table_elems,
                            const __nv_bfloat16* wc_img, const RowEpi& epi, int* status, cudaStream_t st);
 void launch_unpack_rows(const uint8_t* packed, const PackedLayout& pl, int nwindows, float* rows, cudaStream_t st);
-// two-tiles-per-weight-pass QKV projection; b_img: 9 groups x [36][96][8]
-void launch_qkv2(const __nv_bfloat16* a_img, const uint8_t* b_img, int ntiles, __nv_bfloat16* qkv_img,
-                 cudaStream_t st);
 // fused QKV projection + banded attention on window-aligned tiles (Lw == 128); w_img: per (head, rank)
 // [18 k-steps][2][216][8] with rows = [q|k|v] halves
 void launch_qkv_attn(const __nv_bfloat16* a_img, const uint8_t* w_img, int ntiles, int L, int win,
                      __nv_bfloat16* att, cudaStream_t st);
 void launch_attention(const __nv_bfloat16* qkv, __nv_bfloat16* att, int L, int Lw, int win, int nwindows,
                       cudaStream_t st);
-// CTA-pair (cta_group::2) version; w2img is the per-rank half-chunk weight image.
+// fused FFN on CTA pairs (cta_group::2); w2img is the per-rank half-chunk weight image.
 // With wo2img != null the attention out-projection (+ residual, + pre-norm `mid_ln_*` or identity) is
 // fused in front: a_img is then the attention operand image and epi.x the residual before the
 // attention sub-layer.
 void launch_ffn_pair(const __nv_bfloat16* a_img, const uint8_t* w2img, const float* b1, int ff, int ntiles,
                      const RowEpi& epi, cudaStream_t st, const uint8_t* wo2img = nullptr,
                      const float* mid_ln_g = nullptr, const float* mid_ln_b = nullptr);
-void launch_ffn(const __nv_bfloat16* a_img, const uint8_t* w_img, const float* b1, int ff, int ntiles,
-                const RowEpi& epi, cudaStream_t st);
 // The whole encoder stack in one launch (window-aligned tiles, attn_win_size in [1,16]): x is the fp32 residual
 // image written by the embedding kernel.  hp.bases != null: the head (final LayerNorm, fc1, softmax, argmax, Phred,
 // calibration, ASCII) runs in the kernel's tail and x is not written back; otherwise x returns the output of the last

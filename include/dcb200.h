@@ -282,9 +282,10 @@ int dcb_last_forward_ms(dcb_engine* e, float* ms);
 /* Number of engine kernels launched by the last dcb_forward. */
 int dcb_last_forward_launches(dcb_engine* e, int32_t* n);
 
-/* Per-kernel timing of the dominant kernel (the fused FFN): when enabled, every ffn_kernel
- * launch is bracketed by CUDA events on the engine's stream; dcb_get_profile returns the
- * accumulated device time, launch count and tokens processed since dcb_set_profile. */
+/* Per-kernel timing of the dominant kernel (the fused FFN, or the whole encoder stack when it runs
+ * in one launch): when enabled, every ffn_pair_kernel / stack_pair_kernel launch is bracketed by
+ * CUDA events on the engine's stream; dcb_get_profile returns the accumulated device time, launch
+ * count and tokens processed since dcb_set_profile. */
 int dcb_set_profile(dcb_engine* e, int32_t enabled);
 int dcb_get_profile(dcb_engine* e, float* ffn_ms_total, int32_t* ffn_launches, int64_t* ffn_tokens);
 /* Device time (ms) and launch count per kernel class since dcb_set_profile: [0] embed, [1] row GEMM

@@ -15,8 +15,8 @@ extern "C" {
 int dcb_set_debug(dcb_engine* e, int32_t enabled);
 int dcb_debug_residual(dcb_engine* e, int32_t stage, float* out, int64_t out_elems);
 
-/* Developer hook: cycle counters of the last ffn_kernel launch (only meaningful in a -DDCB_TRACE
- * build; 16 uint64 per CTA). */
+/* Developer hook: cycle counters of the last traced kernel launch (the counter buffer is shared by
+ * every kernel with trace hooks; only meaningful in a -DDCB_TRACE build; 16 uint64 per CTA). */
 int dcb_debug_trace(uint64_t* out, int32_t n);
 
 #ifdef __cplusplus

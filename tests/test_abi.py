@@ -46,13 +46,15 @@ def test_config_struct_matches_header_field_order():
   assert names == [f[0] for f in engine.DcbConfig._fields_]
 
 
-def test_product_library_has_no_environment_switches():
-  """The DCB_* kernel-path switches exist only in the developer build."""
+def test_kernel_path_switches_exist_only_in_the_developer_build():
+  """The DCB_* kernel-path switches exist only in the developer build; retired ones exist in neither."""
   prod = open(engine.library_path(), "rb").read()
   dev = open(os.path.join(os.path.dirname(engine.library_path()), "libdcb200_dev.so"), "rb").read()
-  for name in (b"DCB_STACK", b"DCB_FUSE_QA", b"DCB_FFN_PAIR", b"DCB_ALIGN", b"DCB_CHUNK_TILES"):
+  for name in (b"DCB_STACK", b"DCB_FUSE_QA", b"DCB_FUSE_HEAD", b"DCB_ALIGN", b"DCB_CHUNK_TILES"):
     assert name not in prod, name
     assert name in dev, name
+  for name in (b"DCB_QKV2", b"DCB_FFN_PAIR", b"DCB_FFN_CLUSTER"):   # retired switches: neither build reads them
+    assert name not in prod and name not in dev, name
 
 
 def test_no_cpu_fallback_without_gpu():

@@ -515,8 +515,8 @@ def test_initialize_model_from_a_tf_checkpoint(engine_mod, tmp_path):
 
 
 def test_unfused_fallback_paths_agree_with_fused(engine_mod):
-  """DCB_STACK / DCB_FUSE_HEAD / DCB_FUSE_OPROJ / DCB_FUSE_EMBED / DCB_FUSE_QA / DCB_ALIGN / DCB_FFN_PAIR select measured
-  alternatives of the same math.  They exist only in the developer build (libdcb200_dev.so, -DDCB_DEV_SWITCHES) and
+  """DCB_STACK / DCB_FUSE_HEAD / DCB_FUSE_OPROJ / DCB_FUSE_EMBED / DCB_FUSE_QA / DCB_ALIGN select measured alternatives
+  of the same math.  They exist only in the developer build (libdcb200_dev.so, -DDCB_DEV_SWITCHES) and
   are read when an engine is created; the product library ignores the environment (checked first)."""
   p = params_lib.synthetic_params(20, 120, num_hidden_layers=2)
   w = weights_lib.init_weights(p, seed=21)
@@ -528,9 +528,7 @@ def test_unfused_fallback_paths_agree_with_fused(engine_mod):
                     ("per_layer", {"DCB_STACK": "0"}),                  # QKV+attention and out-proj+FFN kernels per layer
                     ("separate_head", {"DCB_FUSE_HEAD": "0"}),          # head_kernel after the stack instead of its fused tail
                     ("unfused", {"DCB_FUSE_OPROJ": "0", "DCB_FUSE_EMBED": "0", "DCB_FUSE_QA": "0"}),
-                    ("packed", {"DCB_ALIGN": "0"}),                     # windows packed back to back, separate QKV / attention
-                    ("single_cta", {"DCB_FFN_PAIR": "0", "DCB_FUSE_QA": "0"}),
-                    ("qkv2", {"DCB_FUSE_QA": "0", "DCB_QKV2": "1"})):
+                    ("packed", {"DCB_ALIGN": "0"})):                    # windows packed back to back, separate QKV / attention
     old = {k: os.environ.get(k) for k in env}
     os.environ.update(env)
     try:
@@ -554,7 +552,6 @@ def test_unfused_fallback_paths_agree_with_fused(engine_mod):
   assert np.abs(outs["fused"] - outs["separate_head"]).max() < 1e-3
   assert np.abs(outs["fused"] - outs["unfused"]).max() < 0.05
   assert np.abs(outs["fused"] - outs["packed"]).max() < 0.05
-  assert np.abs(outs["qkv2"] - outs["unfused"]).max() < 0.05
 
 
 @pytest.mark.parametrize("name", ["rezero_p20", "layernorm_p20", "rezero_p20_bq", "layernorm_p20_bq", "rezero_p5_win3",
